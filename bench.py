@@ -8,6 +8,7 @@ network).  Workload: 16 kHz, block 160, 100 harmonics, 65 noise bands, 4 s, batc
 the N GPUs (strong scaling), reverb 16000 taps, 6 STFT scales.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--workload train|bulk]
+                    [--dump-outputs DIR]
     torchrun --nproc-per-node N bench.py --gpus N ...     (one rank per GPU)
 
 Prints ONE JSON line (rank 0).  `value` = audio samples/s of forward+backward with inputs resident
@@ -49,7 +50,7 @@ BULK_NAME = ("configs[3]: bulk render, 48 kHz, block 512, 256 harmonics, 65 band
 def parse():
     p = argparse.ArgumentParser()
     p.add_argument("--gpus", type=int, default=1)
-    p.add_argument("--steps", type=int, default=100)
+    p.add_argument("--steps", type=int, default=100, help="steps of every timed loop")
     p.add_argument("--warmup", type=int, default=10)
     p.add_argument("--impl", default="b200", choices=["b200", "reference"])
     p.add_argument("--workload", default="train", choices=["train", "bulk"])
@@ -66,7 +67,15 @@ def parse():
     p.add_argument("--skip-configs", action="store_true", help="do not measure the other BASELINE.json configurations")
     p.add_argument("--skip-parity", action="store_true")
     p.add_argument("--bulk-voices", type=int, default=1024, help="voices per GPU of --workload bulk")
-    return p.parse_args()
+    p.add_argument("--dump-outputs", metavar="DIR",
+                   help="after the timed steps, write what the last one computed (audio, loss, gradients; rank 0's voices) "
+                        "as DIR/<name>.npy in float32, so that two builds can be compared output for output")
+    args = p.parse_args()
+    if args.steps < 1:
+        p.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "b200" or args.workload != "train"):
+        p.error("--dump-outputs writes the outputs of --impl b200 --workload train")
+    return args
 
 
 def shapes_module():
@@ -385,6 +394,34 @@ def kernel_table(step, shapes, flush, peaks):
     return rows
 
 
+DUMP_BYTES = 60 << 20          # array data of --dump-outputs: with the .npy headers, under 64 MB in all
+
+
+def step_outputs(step):
+    """What a caller of SynthStep.run() receives: the audio, the loss and the gradient of every leaf."""
+    leaves = ("amp_raw", "dist_raw", "mag_raw", "reverb_noise", "reverb_decay", "reverb_wet")
+    return {"signal": step.signal, "loss": step.loss, **{"grad_" + n: g for n, g in zip(leaves, step.grads)}}
+
+
+def dump_outputs(out_dir, outputs, batch):
+    """Writes each output as out_dir/<name>.npy in float32.  Past DUMP_BYTES the per-voice outputs keep the same fixed,
+    seeded subset of voices, whose indices go to voices.npy."""
+    import numpy as np
+    arrays = {k: v.detach().float().cpu().numpy() for k, v in outputs.items()}
+    per_voice = [k for k in ("signal", "grad_amp_raw", "grad_dist_raw", "grad_mag_raw") if k in arrays]
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_BYTES:
+        voice_bytes = sum(arrays[k].nbytes for k in per_voice) // batch
+        keep = (DUMP_BYTES - total + voice_bytes * batch - 8 * batch) // voice_bytes
+        assert keep >= 1, "a single voice's outputs exceed the dump budget"
+        idx = np.sort(np.random.default_rng(0).choice(batch, keep, replace=False))
+        arrays = {k: a[idx] if k in per_voice else a for k, a in arrays.items()}
+        arrays["voices"] = idx.astype(np.float64)
+    os.makedirs(out_dir, exist_ok=True)
+    for k, a in arrays.items():
+        np.save(os.path.join(out_dir, k + ".npy"), a)
+
+
 def parity_check(step, shapes, host, dev):
     """This run against the float64 oracle, outside the timed region: (a) the first two voices of the benchmark-shape
     step's audio, (b) a two-voice step (same kernels, same reverb) for audio, loss and the reverb-parameter gradients."""
@@ -468,7 +505,7 @@ def run_bulk(args, rank, world):
             dist.barrier()
         torch.cuda.synchronize()
 
-    steps = max(1, min(args.steps, 20))
+    steps = args.steps
     for _ in range(min(args.warmup, 3)):
         r.render(voices)
     barrier()
@@ -571,12 +608,15 @@ def run_b200(args, rank, world):
         graph_note += (" + one eager NCCL all-reduce (AVG) launch on the packed parameter gradients" if args.allreduce_outside
                        else ", the NCCL all-reduce (AVG) of the packed parameter gradients is a node of the graph, "
                             "overlapped with the synthesisers' backward")
+    outputs = None                                  # the captured step's output buffers, rewritten by every replay
     if use_graph:
         try:
             step.capture(forward_only=False)
+            outputs = step_outputs(step)
             step.capture(forward_only=True)
         except Exception as e:                      # stay measurable: fall back to eager launches
             use_graph = False
+            outputs = None
             graph_note = f"eager (graph capture failed: {type(e).__name__})"
             torch.cuda.synchronize()
     else:
@@ -612,6 +652,8 @@ def run_b200(args, rank, world):
             ends[k].record()
         barrier()
         t_wall = time.perf_counter() - t_wall
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, outputs if outputs is not None else step_outputs(step), shapes.batch)
     total_ms = sum(a.elapsed_time(b) for a, b in zip(starts, ends))
     tt = torch.tensor([total_ms], device=dev, dtype=torch.float64)
     if dist is not None:
@@ -621,7 +663,7 @@ def run_b200(args, rank, world):
     value = samples_per_step * args.steps / (total_ms * 1e-3)
 
     # forward only (the "fwd" half of the metric)
-    fwd_ms = event_time(run_fwd, max(10, args.steps // 4), 3, flush)
+    fwd_ms = event_time(run_fwd, args.steps, 3, flush)
     tf = torch.tensor([fwd_ms], device=dev, dtype=torch.float64)
     if dist is not None:
         dist.all_reduce(tf, op=dist.ReduceOp.MAX)
@@ -632,7 +674,7 @@ def run_b200(args, rank, world):
     # launch on that set, and its loss is read back to the host (the read of step k is waited for after step k+1 has
     # been queued, so the host never stalls the device).  Falls back to the staged variant without graphs.
     barrier()
-    e2e_steps = max(10, args.steps // 2)
+    e2e_steps = args.steps
     hosts = [host, {k: v.clone().pin_memory() for k, v in host.items()}]
     paired = use_graph
     link = None
