@@ -17,7 +17,6 @@
 // on both parts independently, so no Hermitian untangling is ever needed.  For the gradient of the
 // filter, sum_pairs G_p * conj(X_p) has the wanted cross-correlation in its real part.
 #include <atomic>
-#include <cstdlib>
 
 #include "fft.cuh"
 #include "regfft.cuh"
@@ -556,23 +555,19 @@ extern "C" int ddsp_b200_twiddle_table(float *table, int n, void *stream) {
 extern "C" int ddsp_b200_conv_plan(int64_t min_len, int *n1, int *n2) {
     DDSP_REQUIRE(n1 && n2 && min_len >= 1);
     // 5-smooth lengths between 2^16 and 2^17: 20 * 4096 and 24 * 4096 (0.625x / 0.75x the work of 2^17)
-    if (!getenv("DDSP_B200_CONV_POW2") && min_len > 65536 && min_len <= 24 * 4096) {
+    if (min_len > 65536 && min_len <= 24 * 4096) {
         *n1 = min_len <= 20 * 4096 ? 20 : 24;
         *n2 = 4096;
         return DDSP_B200_OK;
     }
     int lg = ddsp_ilog2(min_len);
     if (lg < 12) lg = 12;
-    // 128 columns x long rows measured best at 2^17 and 2^18 (tools sweep with DDSP_B200_CONV_LG1: 2^18 bulk render
-    // 10.71 ms with 512 x 512, 10.24 ms with 128 x 2048); rows are capped at 4096 points
+    // 128 columns x long rows measured best at 2^17 and 2^18 (swept with a since-removed split override: 2^18 bulk
+    // render 10.71 ms with 512 x 512, 10.24 ms with 128 x 2048); rows are capped at 4096 points
     int lg1 = lg / 2;
     if (lg1 > 7) lg1 = 7;
     if (lg - lg1 > 12) lg1 = lg - 12;
     if (lg1 > 9) lg1 = 9;
-    if (const char *e = getenv("DDSP_B200_CONV_LG1")) {          // tuning knob: split of the four-step transform
-        const int v = atoi(e);
-        if (v >= 6 && v <= 9 && lg - v >= 6 && lg - v <= 12) lg1 = v;
-    }
     const int lg2 = lg - lg1;
     if (lg2 > 12) return DDSP_B200_EUNSUPPORTED;
     *n1 = 1 << lg1;

@@ -8,16 +8,16 @@
 // Design (DESIGN.md section 3.1).  Only frame-rate controls are read and only audio is written.
 //  * phase: Q0.64 turns.  phi[t] = phase before the first sample of frame t, delta[t] = per-sample
 //    increment; sample j of frame t has phase phi[t] + (j+1)*delta[t]  (inclusive cumsum).
-//  * forward: one thread owns SPT consecutive samples and walks the harmonics with a Reinsch
-//    sine recurrence (2 FMA-pipe ops) + 1 FFMA for the weighted sum; the frame's H weights are
-//    broadcast from shared memory, one LDS.128 per 4 harmonics per SPT samples.  The phase is folded
-//    to |psi| <= pi/2 where the recurrence is stable; the fold's sign (-1)^k goes to two
-//    accumulators (odd / even harmonics).
-//  * backward (d weights): one thread owns (frame, harmonic, chunk of samples) and walks TIME with
+//  * forward: one thread owns 4 consecutive samples of one frame (a frame of bs samples is ceil(bs/4)
+//    such groups; the last one is masked when 4 does not divide bs) and walks the harmonics with a
+//    Reinsch sine recurrence in packed FP32 (FFMA2 / FADD2, two samples per register pair) + 1 FFMA2
+//    for the weighted sum; the frame's H weights sit in shared memory duplicated (A, A), one LDS.128
+//    per 2 harmonics per 4 samples.  The phase is folded to |psi| <= pi/2 where the recurrence is
+//    stable; the fold's sign (-1)^k goes to two accumulators (odd / even harmonics).
+//  * backward (d weights): one thread owns (frame, harmonic pair, chunk of samples) and walks TIME with
 //    the same recurrence (the frame's phase increment is constant), so the reduction over the
 //    frame's samples is a private accumulation; g is broadcast from shared memory.
 #include <cmath>
-#include <cstdlib>
 #include <cstring>
 
 #include "common.cuh"
@@ -115,108 +115,14 @@ phase_scan_kernel(const float *__restrict__ f0, const double *__restrict__ phase
 }
 
 // ------------------------------------------------------------------------------------------
-// Forward.  CTA = FR consecutive frames of one voice; thread = SPT consecutive samples.
+// Forward.  CTA = FR consecutive frames of one voice; work item = (frame, group of 4 consecutive samples), packed FP32
+// (sm_100 FFMA2 / FADD2: one instruction works on a register pair holding two floats).  The group's two sample pairs
+// keep the recurrence state (s, d, u) and the two accumulators in 64-bit registers, weights sit in shared memory already
+// duplicated (A, A) so one LDS.128 feeds two harmonics.  Per harmonic and 4 samples: 6 packed math instructions.
 // ------------------------------------------------------------------------------------------
 constexpr int kFwdThreads = 128;
-constexpr int kFwdMaxThreads = 640;   // packed forward: one sweep of a 16-frame, 160-sample tile (small batches)
+constexpr int kFwdMaxThreads = 640;   // one sweep of a 16-frame, 160-sample tile (small batches)
 
-template <int SPT>
-__global__ void __launch_bounds__(kFwdThreads)
-harmonic_frames_fwd_kernel(const float *__restrict__ weights, const uint64_t *__restrict__ phi,
-                           const uint64_t *__restrict__ delta, float *__restrict__ audio, int T,
-                           int H, int Hp, int bs, int FR) {
-    extern __shared__ __align__(16) float smem[];
-    float *w = smem;                                          // [FR][Hp], zero padded to Hp
-    uint64_t *sphi = reinterpret_cast<uint64_t *>(w + (size_t)FR * Hp);   // [FR]
-    uint64_t *sdel = sphi + FR;                               // [FR]
-
-    const int b = blockIdx.y;
-    const int t0 = blockIdx.x * FR;
-    const int nfr = min(FR, T - t0);
-    const int tid = threadIdx.x;
-
-    const float *wg = weights + ((size_t)b * T + t0) * H;
-    for (int i = tid; i < nfr * Hp; i += kFwdThreads) {
-        int f = i / Hp, k = i - f * Hp;
-        w[i] = k < H ? __ldg(wg + (size_t)f * H + k) : 0.f;
-    }
-    if (tid < nfr) {
-        sphi[tid] = phi[(size_t)b * T + t0 + tid];
-        sdel[tid] = delta[(size_t)b * T + t0 + tid];
-    }
-    __syncthreads();
-
-    const int S = nfr * bs;
-    float *out = audio + ((size_t)b * T + t0) * bs;
-    for (int i0 = tid * SPT; i0 < S; i0 += kFwdThreads * SPT) {
-        const int f = i0 / bs;
-        const int j0 = i0 - f * bs;                // SPT | bs, so the SPT samples share frame f
-        const uint64_t ph = sphi[f], dl = sdel[f];
-        const float4 *wr = reinterpret_cast<const float4 *>(w + (size_t)f * Hp);
-
-        ddsp_osc o[SPT];
-        float q[SPT], ch[SPT], ae[SPT], ao[SPT];
-        int flip[SPT];
-#pragma unroll
-        for (int s = 0; s < SPT; ++s) {
-            uint64_t p = ph + (uint64_t)(j0 + s + 1) * dl;
-            float x = ddsp_fold_quarter(p, &flip[s]) * DDSP_PI_F;   // psi/2 in radians
-            float sh = ddsp_sin_q(x);
-            ch[s] = ddsp_cos_q(x);
-            q[s] = 2.f * sh;
-            o[s].u = -q[s] * q[s];
-            o[s].s = q[s] * ch[s];                 // sin(psi)
-            o[s].d = o[s].s;                       // s_1 - s_0
-            ae[s] = 0.f;
-            ao[s] = 0.f;
-        }
-        for (int k0 = 0; k0 < Hp; k0 += kReseed) {
-            if (k0 > 0) {
-                // exact re-seed at harmonic k = k0+1 from the fixed-point phase
-#pragma unroll
-                for (int s = 0; s < SPT; ++s) {
-                    uint64_t p = ph + (uint64_t)(j0 + s + 1) * dl;
-                    uint32_t r = (uint32_t)(((p >> 62) + 1) >> 1);
-                    uint64_t psi = p - ((uint64_t)r << 63);
-                    float a = ddsp_turns_signed((uint64_t)(k0 + 1) * psi) * DDSP_2PI_F;
-                    float sk, ck;
-                    __sincosf(a, &sk, &ck);
-                    o[s].s = sk;
-                    // s_k - s_{k-1} = 2 sin(psi/2) cos((k-1/2) psi)
-                    o[s].d = q[s] * fmaf(ck, ch[s], sk * (0.5f * q[s]));
-                }
-            }
-            const int kend = min(k0 + kReseed, Hp);
-            for (int k = k0; k < kend; k += 4) {
-                const float4 a = wr[k >> 2];
-#pragma unroll
-                for (int s = 0; s < SPT; ++s) {
-                    ao[s] = fmaf(a.x, o[s].s, ao[s]); o[s].step();
-                    ae[s] = fmaf(a.y, o[s].s, ae[s]); o[s].step();
-                    ao[s] = fmaf(a.z, o[s].s, ao[s]); o[s].step();
-                    ae[s] = fmaf(a.w, o[s].s, ae[s]); o[s].step();
-                }
-            }
-        }
-        float y[SPT];
-#pragma unroll
-        for (int s = 0; s < SPT; ++s) y[s] = flip[s] ? ae[s] - ao[s] : ae[s] + ao[s];
-        if (SPT == 4) {
-            *reinterpret_cast<float4 *>(out + i0) = make_float4(y[0], y[1], y[2], y[3]);
-        } else if (SPT == 2) {
-            *reinterpret_cast<float2 *>(out + i0) = make_float2(y[0], y[1]);
-        } else {
-            out[i0] = y[0];
-        }
-    }
-}
-
-// ------------------------------------------------------------------------------------------
-// Forward, packed-FP32 variant (sm_100 FFMA2 / FADD2: one instruction works on a register pair holding
-// two floats).  Thread = 4 consecutive samples = two pairs; the recurrence state (s, d, u) and the two
-// accumulators live in 64-bit registers, weights sit in shared memory already duplicated (A, A) so one
-// LDS.128 feeds two harmonics.  Per harmonic and 4 samples: 6 packed math instructions instead of 12.
-// ------------------------------------------------------------------------------------------
 // RAW: the CTA's weights are not read but computed from the control net's raw outputs in the prologue --
 // HarmonicSynth.get_controls (modules.py:44-67: scale_function on both, Nyquist mask, normalise) and the in-place
 // `distribution *= amplitudes` of modules.py:73, with the arithmetic of controls_fwd_kernel (bit-identical results);
@@ -332,11 +238,11 @@ harmonic_frames_fwd_x2_kernel(const float *__restrict__ weights, const uint64_t 
         __syncthreads();
     }
 
-    const int S = nfr * bs;
+    const int G = (bs + 3) >> 2;                          // groups per frame (4 | bs: item it = the CTA's samples 4it..4it+3)
     float *out = audio + ((size_t)b * T + t0) * bs;
-    for (int i0 = tid * 4; i0 < S; i0 += nthr * 4) {
-        const int f = i0 / bs;
-        const int j0 = i0 - f * bs;
+    for (int it = tid; it < nfr * G; it += nthr) {
+        const int f = it / G;
+        const int j0 = 4 * (it - f * G);
         const uint64_t ph = sphi[f], dl = sdel[f];
         const ulonglong2 *wr = reinterpret_cast<const ulonglong2 *>(w2 + (size_t)f * Hp);   // 2 harmonics each
 
@@ -391,81 +297,27 @@ harmonic_frames_fwd_x2_kernel(const float *__restrict__ weights, const uint64_t 
         float ae[4], ao[4];
         unpk2(aeA, ae[0], ae[1]); unpk2(aeB, ae[2], ae[3]);
         unpk2(aoA, ao[0], ao[1]); unpk2(aoB, ao[2], ao[3]);
-        float4 y;
-        y.x = flip[0] ? ae[0] - ao[0] : ae[0] + ao[0];
-        y.y = flip[1] ? ae[1] - ao[1] : ae[1] + ao[1];
-        y.z = flip[2] ? ae[2] - ao[2] : ae[2] + ao[2];
-        y.w = flip[3] ? ae[3] - ao[3] : ae[3] + ao[3];
-        *reinterpret_cast<float4 *>(out + i0) = y;
+        float y[4];
+#pragma unroll
+        for (int e = 0; e < 4; ++e) y[e] = flip[e] ? ae[e] - ao[e] : ae[e] + ao[e];
+        float *o = out + (size_t)f * bs + j0;
+        if ((bs & 3) == 0) {
+            *reinterpret_cast<float4 *>(o) = make_float4(y[0], y[1], y[2], y[3]);
+        } else {                                          // frames start unaligned; the last group is masked
+#pragma unroll
+            for (int e = 0; e < 4; ++e)
+                if (j0 + e < bs) o[e] = y[e];
+        }
     }
 }
 
 // ------------------------------------------------------------------------------------------
-// Backward w.r.t. weights.  CTA = FR frames of one voice; work item = (chunk, frame, harmonic).
+// Backward w.r.t. weights.  CTA = FR frames of one voice; work item = (chunk, frame, harmonic pair).
 // ------------------------------------------------------------------------------------------
 constexpr int kBwdThreads = 256;
 
-__global__ void __launch_bounds__(kBwdThreads)
-harmonic_frames_bwd_w_kernel(const float *__restrict__ g_audio, const uint64_t *__restrict__ phi,
-                             const uint64_t *__restrict__ delta, float *__restrict__ d_weights,
-                             int T, int H, int bs, int FR, int nchunk, int clen) {
-    extern __shared__ __align__(16) float smem[];
-    float *g = smem;                                   // [FR*bs]
-    float *part = g + (((size_t)FR * bs + 3) & ~(size_t)3);   // [nchunk][FR][H]
-    const int b = blockIdx.y;
-    const int t0 = blockIdx.x * FR;
-    const int nfr = min(FR, T - t0);
-    const int tid = threadIdx.x;
-
-    const float *gg = g_audio + ((size_t)b * T + t0) * bs;
-    for (int i = tid; i < nfr * bs; i += kBwdThreads) g[i] = __ldg(gg + i);
-    __syncthreads();
-
-    const int items = nchunk * nfr * H;
-    for (int it = tid; it < items; it += kBwdThreads) {
-        const int k = it % H;                          // harmonic index k+1; fastest -> g broadcasts
-        const int fc = it / H;
-        const int f = fc % nfr;
-        const int c = fc / nfr;
-        const int jlo = c * clen, jhi = min(jlo + clen, bs);
-        const uint64_t ph = phi[(size_t)b * T + t0 + f], dl = delta[(size_t)b * T + t0 + f];
-        const uint64_t kk = (uint64_t)(k + 1);
-        // per-sample rotation of harmonic k: alpha = k*delta, folded to [-1/4,1/4) + parity
-        const uint64_t alpha = kk * dl;
-        const uint32_t r = (uint32_t)(((alpha >> 62) + 1) >> 1);
-        const uint64_t af = alpha - ((uint64_t)r << 63);
-        const float xa = ddsp_turns_signed(af) * DDSP_PI_F;          // alpha_f/2 in radians
-        const float q = 2.f * ddsp_sin_q(xa);
-        ddsp_osc o;
-        o.u = -q * q;
-        // phase of the chunk's first sample
-        const uint64_t th = kk * (ph + (uint64_t)(jlo + 1) * dl);
-        o.s = __sinf(ddsp_turns_signed(th) * DDSP_2PI_F);
-        // s_0 - s_{-1} = 2 sin(alpha_f/2) cos(theta - alpha_f/2)
-        o.d = q * __cosf(ddsp_turns_signed(th - (uint64_t)((int64_t)af >> 1)) * DDSP_2PI_F);
-        const float *gp = g + (size_t)f * bs;
-        float a0 = 0.f, a1 = 0.f;                      // even / odd offsets from jlo
-        int j = jlo;
-        for (; j + 1 < jhi; j += 2) {
-            a0 = fmaf(gp[j], o.s, a0);
-            o.step();
-            a1 = fmaf(gp[j + 1], o.s, a1);
-            o.step();
-        }
-        if (j < jhi) a0 = fmaf(gp[j], o.s, a0);
-        part[((size_t)c * nfr + f) * H + k] = (r & 1u) ? a0 - a1 : a0 + a1;
-    }
-    __syncthreads();
-    float *dw = d_weights + ((size_t)b * T + t0) * H;
-    for (int i = tid; i < nfr * H; i += kBwdThreads) {
-        float acc = 0.f;
-        for (int c = 0; c < nchunk; ++c) acc += part[(size_t)c * nfr * H + i];
-        dw[i] = acc;
-    }
-}
-
-// Backward w.r.t. weights, packed-FP32 variant: one thread walks time for TWO harmonics (k, k+1) held in
-// a register pair; g is staged duplicated (g, g) so the packed FFMA2 needs no per-step packing.
+// Packed FP32: one thread walks time for TWO harmonics (k, k+1) held in a register pair; g is staged
+// duplicated (g, g) so the packed FFMA2 needs no per-step packing.
 // RAW: the chunk partials are not written out as d_weights but taken through the backward of the controls
 // (controls_bwd_kernel's arithmetic with d_amps = d_dist = 0) in the epilogue, one warp per frame row: the gradient
 // arrives at the control net's raw outputs in the same launch.
@@ -818,7 +670,7 @@ extern "C" int ddsp_b200_phase_scan(const float *f0, const double *phase0, uint6
 }
 
 // frames per CTA: the smallest count that makes the CTA's samples a whole number of
-// (threads x SPT) sweeps, so no thread idles in the last sweep (bs=160 -> 16 frames, 512 -> 1)
+// (threads x 4) sweeps, so no thread idles in the last sweep (bs=160 -> 16 frames, 512 -> 1)
 static int frames_per_cta(int bs, int T, int sweep, int cap) {
     int fr = 1;
     while (fr < cap && (fr * bs) % sweep != 0) ++fr;
@@ -827,53 +679,32 @@ static int frames_per_cta(int bs, int T, int sweep, int cap) {
     return fr < 1 ? 1 : fr;
 }
 
-// shared by the two forward entry points; rc = nullptr: weights are read, else computed in the prologue (x2 kernel only)
+// shared by the two forward entry points; rc = nullptr: weights are read, else computed in the prologue
 static int launch_frames_fwd(const float *weights, const RawControls *rc, const uint64_t *phi, const uint64_t *delta,
                              float *audio, int B, int T, int H, int block_size, cudaStream_t st) {
     const int bs = block_size;
-    const int spt = (bs % 4 == 0) ? 4 : (bs % 2 == 0) ? 2 : 1;
+    const int bsp = (bs + 3) & ~3;                                      // frame length in whole groups of 4 samples
     const int Hp = (H + 3) & ~3;
-    const int fr = frames_per_cta(bs, T, kFwdThreads * spt, 32);
-    const size_t smem = (size_t)fr * Hp * sizeof(float) + 2 * (size_t)fr * sizeof(uint64_t);
+    int fr = frames_per_cta(bsp, T, kFwdThreads * 4, 32);
+    auto bytes = [&](int fr_) { return 2 * (size_t)fr_ * Hp * sizeof(float) + 2 * (size_t)fr_ * sizeof(uint64_t); };
+    while (bytes(fr) > 200 * 1024 && fr > 1) fr = (fr + 1) / 2;
+    const size_t smem = bytes(fr);
+    // one frame's (A, A) table must fit: H <= 25 596, far above the harmonics the Nyquist mask keeps at 1 Hz / 48 kHz
     if (smem > 200 * 1024) return DDSP_B200_EUNSUPPORTED;
+    if (rc && H > 256) return DDSP_B200_EUNSUPPORTED;
     dim3 grid((T + fr - 1) / fr, B);
-#define LAUNCH(SPT)                                                                              \
-    do {                                                                                         \
-        if (smem > 48 * 1024)                                                                    \
-            cudaFuncSetAttribute(harmonic_frames_fwd_kernel<SPT>,                                \
-                                 cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);        \
-        harmonic_frames_fwd_kernel<SPT><<<grid, kFwdThreads, smem, st>>>(weights, phi, delta,    \
-                                                                         audio, T, H, Hp, bs, fr); \
-    } while (0)
-    static const bool scalar_only = getenv("DDSP_B200_HARMONIC_SCALAR") != nullptr;   // A/B switch
-    const size_t smem2 = 2 * (size_t)fr * Hp * sizeof(float) + 2 * (size_t)fr * sizeof(uint64_t);
-    const bool packed = spt == 4 && smem2 <= 200 * 1024 && (rc || !scalar_only);
-    if (rc && (!packed || H > 256)) return DDSP_B200_EUNSUPPORTED;
-    if (packed) {
-        // few voices (strong scaling leaves 8 per GPU, realtime 1): the grid alone leaves most warp slots empty, so
-        // the CTA takes more threads = fewer sweeps per thread, until about 16 warps per SM are in flight
-        int threads = kFwdThreads;
-        const long long ctas = (long long)grid.x * grid.y;
-        const int max_useful = (int)(((long long)fr * bs / 4 + 31) / 32 * 32);          // one sweep covers the tile
-        while (threads < kFwdMaxThreads && threads < max_useful && ctas * (threads / 32) < 16ll * DDSP_SM_COUNT)
-            threads += kFwdThreads;
-        if (threads > max_useful) threads = max_useful > kFwdThreads ? max_useful : kFwdThreads;
-        if (threads > kFwdMaxThreads) threads = kFwdMaxThreads;
-        if (rc) {
-            if (smem2 > 48 * 1024)
-                cudaFuncSetAttribute(harmonic_frames_fwd_x2_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                     (int)smem2);
-            harmonic_frames_fwd_x2_kernel<true><<<grid, threads, smem2, st>>>(nullptr, phi, delta, audio, T, H, Hp, bs,
-                                                                               fr, *rc);
-        } else {
-            if (smem2 > 48 * 1024)
-                cudaFuncSetAttribute(harmonic_frames_fwd_x2_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                     (int)smem2);
-            harmonic_frames_fwd_x2_kernel<false><<<grid, threads, smem2, st>>>(weights, phi, delta, audio, T, H, Hp, bs,
-                                                                                fr, RawControls{});
-        }
-    } else if (spt == 4) LAUNCH(4); else if (spt == 2) LAUNCH(2); else LAUNCH(1);
-#undef LAUNCH
+    // few voices (strong scaling leaves 8 per GPU, realtime 1): the grid alone leaves most warp slots empty, so
+    // the CTA takes more threads = fewer sweeps per thread, until about 16 warps per SM are in flight
+    int threads = kFwdThreads;
+    const long long ctas = (long long)grid.x * grid.y;
+    const int max_useful = (int)(((long long)fr * bsp / 4 + 31) / 32 * 32);         // one sweep covers the tile
+    while (threads < kFwdMaxThreads && threads < max_useful && ctas * (threads / 32) < 16ll * DDSP_SM_COUNT)
+        threads += kFwdThreads;
+    if (threads > max_useful) threads = max_useful > kFwdThreads ? max_useful : kFwdThreads;
+    if (threads > kFwdMaxThreads) threads = kFwdMaxThreads;
+    auto kernel = rc ? harmonic_frames_fwd_x2_kernel<true> : harmonic_frames_fwd_x2_kernel<false>;
+    if (smem > 48 * 1024) cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    kernel<<<grid, threads, smem, st>>>(weights, phi, delta, audio, T, H, Hp, bs, fr, rc ? *rc : RawControls{});
     return ddsp_launch_status();
 }
 
@@ -935,43 +766,24 @@ static int launch_frames_bwd(const float *g_audio, const uint64_t *phi, const ui
     const int bs = block_size;
     const int nchunk = (bs + kChunk - 1) / kChunk;
     const int clen = (((bs + nchunk - 1) / nchunk) + 1) & ~1;   // even, so chunk parity is uniform
-    static const bool scalar_only = getenv("DDSP_B200_HARMONIC_SCALAR") != nullptr;   // A/B switch
-    const bool packed = rc || !scalar_only;
-    const int per_frame = nchunk * (packed ? (H + 1) / 2 : H);          // work items per frame
-    // enough (chunk, frame, harmonic) items for >= 4 sweeps of the CTA
+    const int per_frame = nchunk * ((H + 1) / 2);                  // work items per frame
+    // enough (chunk, frame, harmonic pair) items for >= 4 sweeps of the CTA
     int fr = (4 * kBwdThreads + per_frame - 1) / per_frame;
     if (fr > T) fr = T;
     if (fr < 1) fr = 1;
     auto bytes = [&](int fr_) {
-        const size_t gsz = packed ? 2 * (((size_t)fr_ * bs + 1) & ~(size_t)1) : (((size_t)fr_ * bs + 3) & ~(size_t)3);
+        const size_t gsz = 2 * (((size_t)fr_ * bs + 1) & ~(size_t)1);
         return (gsz + (size_t)nchunk * fr_ * H + (rc ? 2 * (size_t)fr_ * H : 0)) * sizeof(float);
     };
     while (bytes(fr) > 200 * 1024 && fr > 1) fr = (fr + 1) / 2;
     const size_t smem = bytes(fr);
     if (smem > 200 * 1024) return DDSP_B200_EUNSUPPORTED;
+    if (rc && H > 256) return DDSP_B200_EUNSUPPORTED;
     dim3 grid((T + fr - 1) / fr, B);
-    if (rc) {
-        if (H > 256) return DDSP_B200_EUNSUPPORTED;
-        if (smem > 48 * 1024)
-            cudaFuncSetAttribute(harmonic_frames_bwd_w_x2_kernel<true>,
-                                 cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-        harmonic_frames_bwd_w_x2_kernel<true><<<grid, kBwdThreads, smem, st>>>(g_audio, phi, delta, nullptr, T, H, bs, fr,
-                                                                               nchunk, clen, *rc);
-        return ddsp_launch_status();
-    }
-    if (packed) {
-        if (smem > 48 * 1024)
-            cudaFuncSetAttribute(harmonic_frames_bwd_w_x2_kernel<false>,
-                                 cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-        harmonic_frames_bwd_w_x2_kernel<false><<<grid, kBwdThreads, smem, st>>>(g_audio, phi, delta, d_weights, T, H, bs,
-                                                                                fr, nchunk, clen, RawControlsGrad{});
-        return ddsp_launch_status();
-    }
-    if (smem > 48 * 1024)
-        cudaFuncSetAttribute(harmonic_frames_bwd_w_kernel,
-                             cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    harmonic_frames_bwd_w_kernel<<<grid, kBwdThreads, smem, st>>>(g_audio, phi, delta, d_weights, T, H, bs, fr, nchunk,
-                                                                  clen);
+    auto kernel = rc ? harmonic_frames_bwd_w_x2_kernel<true> : harmonic_frames_bwd_w_x2_kernel<false>;
+    if (smem > 48 * 1024) cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    kernel<<<grid, kBwdThreads, smem, st>>>(g_audio, phi, delta, d_weights, T, H, bs, fr, nchunk, clen,
+                                            rc ? *rc : RawControlsGrad{});
     return ddsp_launch_status();
 }
 

@@ -28,7 +28,6 @@
 //     64 KB of L1 for the sample re-reads (a pair re-reads 12 of its predecessor's 20 slots), the window and the stage
 //     twiddles.
 //   * mss_combine2_kernel sums the scales in order and folds the reflect padding back.
-#include <cstdlib>
 
 #include "common.cuh"
 #include "pfft.cuh"
@@ -496,8 +495,7 @@ int make_plan(int B, int64_t N, const int *scales, int n_scales, Plan2 *out) {
     long long off = 0, pairs = 0;
     int item = 0, max_hop = 0;
     // about 16 tiles per resident CTA slot in total, shared evenly by the scales (their work is about equal)
-    long long per_slot = 16;                 // measured: 4..32 are within 2 % of each other at batch 64
-    if (const char *e = getenv("DDSP_B200_MSS_TILES_PER_SLOT")) per_slot = atoi(e) > 0 ? atoi(e) : per_slot;   // tuning knob
+    const long long per_slot = 16;           // measured: 4..32 are within 2 % of each other at batch 64
     const long long want_tiles = ddsp_ceil_div(per_slot * 2 * DDSP_SM_COUNT, (long long)n_scales * B);
     for (int i = 0; i < n_scales; ++i) {
         const int s = scales[i];

@@ -72,7 +72,8 @@ uint64_t ddsp_b200_pitch_to_q64(float f0, double sample_rate);
 int ddsp_b200_phase_scan(const float *f0, const double *phase0, uint64_t *phi, uint64_t *delta,
                          double *phase_end, int B, int T, int block_size, double sample_rate,
                          void *stream);
-/* weights[B,T,H] = harmonic_distribution * amplitudes;  audio[B, T*bs]. */
+/* weights[B,T,H] = harmonic_distribution * amplitudes;  audio[B, T*bs].  Any block_size; H <= 25 596 (one frame's
+ * weights, duplicated, in shared memory), else DDSP_B200_EUNSUPPORTED. */
 int ddsp_b200_harmonic_frames_fwd(const float *weights, const uint64_t *phi, const uint64_t *delta,
                                   float *audio, int B, int T, int H, int block_size, void *stream);
 /* d_weights[B,T,H] = sum over the frame's samples of g * sin(k*phase). */

@@ -174,21 +174,22 @@ def test_harmonic_frames_config1_shapes(ddsp, orc):
 
 
 def test_harmonic_frames_config4_shapes_and_reseed(ddsp, orc):
-    """48 kHz, block 512, 256 harmonics (crosses the recurrence re-seed at harmonic 129)."""
+    """48 kHz, block 512, 256 harmonics (crosses the recurrence re-seed at harmonic 129); and 2000 harmonics at
+    block 160, a weight table too large for 16 frames per CTA (the forward takes fewer frames per CTA)."""
     gen = torch.Generator().manual_seed(4)
-    B, T, bs, H, sr = 1, 24, 512, 256, 48000
-    f0 = torch.rand(B, T, 1, generator=gen) * 120 + 40
-    w = torch.rand(B, T, H, generator=gen) * (2.0 / H)
-    ref = orc.harmonic_synth(orc.upsample(f0.double(), bs), orc.upsample(w.double(), bs), sr)
-    wd = w.cuda().requires_grad_(True)
-    got, _ = ddsp.harmonic_synth_frames(f0.cuda(), wd, bs, sr)
-    assert_audio(got, ref)
-    go = torch.randn(B, T * bs, 1, generator=gen)
-    (got * go.cuda()).sum().backward()
-    w64 = w.double().requires_grad_(True)
-    y = orc.harmonic_synth(orc.upsample(f0.double(), bs), orc.upsample(w64, bs), sr)
-    (y * go.double()).sum().backward()
-    assert_grad(wd.grad, w64.grad)
+    for B, T, bs, H, sr in ((1, 24, 512, 256, 48000), (1, 20, 160, 2000, 16000)):
+        f0 = torch.rand(B, T, 1, generator=gen) * 120 + 40
+        w = torch.rand(B, T, H, generator=gen) * (2.0 / H)
+        ref = orc.harmonic_synth(orc.upsample(f0.double(), bs), orc.upsample(w.double(), bs), sr)
+        wd = w.cuda().requires_grad_(True)
+        got, _ = ddsp.harmonic_synth_frames(f0.cuda(), wd, bs, sr)
+        assert_audio(got, ref)
+        go = torch.randn(B, T * bs, 1, generator=gen)
+        (got * go.cuda()).sum().backward()
+        w64 = w.double().requires_grad_(True)
+        y = orc.harmonic_synth(orc.upsample(f0.double(), bs), orc.upsample(w64, bs), sr)
+        (y * go.double()).sum().backward()
+        assert_grad(wd.grad, w64.grad)
 
 
 def test_harmonic_frames_odd_block_and_streaming(ddsp, orc):
@@ -667,6 +668,8 @@ def test_unsupported_shapes_fail_loudly(ddsp):
         ddsp.multiscale_fft(torch.rand(1, 100).cuda(), [512], 0.75)
     with pytest.raises(RuntimeError):           # float64 is the oracle's job
         ddsp.scale_function(torch.zeros(4, dtype=torch.float64).cuda())
+    with pytest.raises(RuntimeError):           # one frame's duplicated weights exceed shared memory
+        ddsp.harmonic_synth_frames(torch.full((1, 1, 1), 100.0).cuda(), torch.rand(1, 1, 30000).cuda(), 160, 16000)
 
 
 def test_large_amplitude_and_extreme_pitch(ddsp, orc):
