@@ -27,7 +27,7 @@ __all__ = [
     "safe_log", "mean_std_loudness", "multiscale_fft", "resample", "upsample", "remove_above_nyquist",
     "scale_function", "extract_loudness", "extract_pitch", "mlp", "gru", "harmonic_synth",
     "amp_to_impulse_response", "fft_convolve",
-    "harmonic_synth_frames", "filtered_noise", "multiscale_spectral_loss",
+    "harmonic_synth_frames", "filtered_noise", "multiscale_spectral_loss", "convolve_stream",
 ]
 
 
@@ -288,6 +288,20 @@ def harmonic_synth_from_raw(first, dist_raw, f0, block_size: int, sample_rate, p
 def filtered_noise(magnitudes, noise):
     """Extension: FilteredNoise.forward with the uniform(-1,1) draw passed in (B,T,block)."""
     return _F.FilteredNoise.apply(magnitudes, noise)
+
+
+def convolve_stream(signal, kernel, history: Optional[torch.Tensor] = None):
+    """Extension: one buffer of a causal convolution that continues across calls (Reverb.forward, modules.py:28-35,
+    played buffer by buffer).  signal (B,N), kernel with L taps (L elements, e.g. (L,) or (1,L) or the reverb's
+    (1,L,1) impulse), history (B,L-1) = the previous L-1 input samples, oldest first; None = silence before.
+    -> (out (B,N), history (B,L-1) for the next call).  out[b,n] = sum_k kernel[k] * [history | signal][b, L-1+n-k].
+    Direct form, B*N*L FMA.  Forward only: inputs that require grad raise under grad mode."""
+    L = kernel.numel()
+    if history is None:
+        history = signal.new_zeros(signal.shape[0], max(L - 1, 0))
+    if torch.is_grad_enabled() and any(t.requires_grad for t in (signal, kernel, history)):
+        raise RuntimeError("convolve_stream has no backward: call it under torch.no_grad() or on detached tensors")
+    return _F._ops.conv_stream_fwd(signal, kernel, history)
 
 
 def multiscale_spectral_loss(target, rec, scales: Sequence[int], overlap: float):

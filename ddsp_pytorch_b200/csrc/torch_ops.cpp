@@ -664,6 +664,27 @@ std::tuple<Tensor, Tensor, Tensor> reverb_impulse_bwd(const Tensor &d_imp_, cons
     return {dn, dd, dw};
 }
 
+// ---------------------------------------------------------------------------------------- a10s streaming reverb
+// signal (B,N), kernel with L taps (any shape of L elements), history (B,L-1) -> (y (B,N), history_out (B,L-1))
+std::tuple<Tensor, Tensor> conv_stream_fwd(const Tensor &signal_, const Tensor &kernel_, const Tensor &history_) {
+    Tensor sig = prep(signal_, "signal"), ker = prep(kernel_, "kernel"), hist = prep(history_, "history");
+    TORCH_CHECK(sig.dim() == 2 && sig.size(0) >= 1 && sig.size(1) >= 1, "conv_stream: signal must be (B,N), B, N >= 1");
+    const int64_t B = sig.size(0), N = sig.size(1), L = ker.numel();
+    TORCH_CHECK(L >= 1 && L <= INT32_MAX && B <= INT32_MAX, "conv_stream: the kernel needs 1 .. 2^31-1 taps");
+    TORCH_CHECK(hist.dim() == 2 && hist.size(0) == B && hist.size(1) == L - 1, "conv_stream: history must be (B, L-1) = (",
+                B, ", ", L - 1, "), got ", hist.sizes());
+    TORCH_CHECK(ker.device() == sig.device() && hist.device() == sig.device(), "conv_stream: tensors on different devices");
+    c10::cuda::CUDAGuard guard(sig.device());
+    Tensor y = at::empty_like(sig), hist_out = at::empty_like(hist);
+    const int64_t ns = ddsp_b200_conv_stream_scratch((int)B, N, (int)L);       // sizes checked above: >= 0
+    Tensor scratch = ns > 0 ? at::empty({ns}, sig.options()) : Tensor();
+    check(ddsp_b200_conv_stream_fwd(fp(sig), fp(ker), L > 1 ? fp(hist) : nullptr, fpm(y),
+                                    L > 1 ? fpm(hist_out) : nullptr, (int)B, N, (int)L,
+                                    ns > 0 ? fpm(scratch) : nullptr, cur_stream()),
+          "conv_stream_fwd");
+    return {y, hist_out};
+}
+
 // ---------------------------------------------------------------------------------------- a11, a12
 int64_t pow2_ge(int64_t v) {
     int64_t p = 1;
@@ -981,6 +1002,7 @@ TORCH_LIBRARY(ddsp_b200, m) {
     m.def("fftconv_bwd_parts(Tensor grad_out, Tensor signal, Tensor kernel, Tensor? work_x, Tensor? hspec, Tensor? work_g, bool need_signal, bool need_kernel) -> (Tensor, Tensor, Tensor)");
     m.def("reverb_impulse_fwd(Tensor noise, Tensor decay, Tensor wet, Tensor t) -> Tensor");
     m.def("reverb_impulse_bwd(Tensor d_impulse, Tensor noise, Tensor decay, Tensor wet, Tensor t) -> (Tensor, Tensor, Tensor)");
+    m.def("conv_stream_fwd(Tensor signal, Tensor kernel, Tensor history) -> (Tensor, Tensor)");
     m.def("stft_mag_fwd(Tensor signal, Tensor window, int n_fft, int hop) -> Tensor");
     m.def("stft_mag_bwd(Tensor signal, Tensor d_mag, Tensor window, int n_fft, int hop) -> Tensor");
     m.def("mss_loss_fwd(Tensor target, Tensor rec, int[] scales, float overlap, Tensor windows, bool need_grad) -> (Tensor, Tensor)");
@@ -1016,6 +1038,7 @@ TORCH_LIBRARY_IMPL(ddsp_b200, CUDA, m) {
     m.impl("fftconv_bwd_parts", fftconv_bwd_parts);
     m.impl("reverb_impulse_fwd", reverb_impulse_fwd);
     m.impl("reverb_impulse_bwd", reverb_impulse_bwd);
+    m.impl("conv_stream_fwd", conv_stream_fwd);
     m.impl("stft_mag_fwd", stft_mag_fwd);
     m.impl("stft_mag_bwd", stft_mag_bwd);
     m.impl("mss_loss_fwd", mss_loss_fwd);

@@ -10,8 +10,10 @@ with the dataset mean/std, inputs strided to frame rate by ``block_size``) whose
 
 Streaming state lives in buffers: the GRU hidden state (``cache_gru``, as the reference) and the
 oscillator phase (``phase``: the reference registers it at decoder.py:99 and never uses it, so every
-1024-sample buffer restarted the phase at zero).  The C++ host must load ``libddsp_b200_torch.so`` before
-``torch::jit::load`` (INTEGRATION.md section 4).
+1024-sample buffer restarted the phase at zero).  A realtime export is dry by default; with
+``streaming_reverb=True`` it also plays the trained reverb, carrying the last L-1 samples of the reverb's input
+in ``reverb_history`` so that the impulse's tail runs on into the following buffers.  The C++ host must load
+``libddsp_b200_torch.so`` before ``torch::jit::load`` (INTEGRATION.md section 4).
 """
 from __future__ import annotations
 
@@ -27,11 +29,13 @@ from .models.decoder import DDSPDecoder
 class ScriptDDSP(nn.Module):
     # compile-time constants: the scripted graph only contains the branches that are taken
     __constants__ = ["block_size", "sample_rate", "reverb_length", "has_reverb", "realtime", "device_noise",
-                     "mean_loudness", "std_loudness", "noise_bias", "cluster_gru"]
+                     "mean_loudness", "std_loudness", "noise_bias", "cluster_gru", "streaming_reverb"]
 
     def __init__(self, ddsp: DDSPDecoder, mean_loudness: float, std_loudness: float, realtime: bool = True,
-                 device_noise: bool = True):
+                 device_noise: bool = True, streaming_reverb: bool = False):
         super().__init__()
+        if streaming_reverb and not (realtime and ddsp.has_reverb):
+            raise ValueError("streaming_reverb needs realtime=True and a model built with has_reverb=True")
         dec = ddsp.decoder
         assert not dec.add_z, "export covers the f0 + loudness decoder (config.yaml's single-inst-decoder)"
         self.f0_mlp = dec.f0_mlp
@@ -55,6 +59,11 @@ class ScriptDDSP(nn.Module):
         self.sample_rate: float = float(ddsp.sample_rate)
         self.reverb_length: int = int(ddsp.reverb.length)
         self.has_reverb: bool = bool(ddsp.has_reverb) and not realtime     # the host convolves (patches/example.pd)
+        # realtime reverb: the last L-1 samples of the reverb's input, batch 1 like cache_gru and phase
+        self.streaming_reverb: bool = bool(streaming_reverb)
+        if self.streaming_reverb:
+            self.register_buffer("reverb_history", torch.zeros(1, self.reverb_length - 1,
+                                                               device=ddsp.reverb.noise.device))
         self.realtime: bool = realtime
         self.device_noise: bool = device_noise
         self.mean_loudness: float = float(mean_loudness)
@@ -112,19 +121,30 @@ class ScriptDDSP(nn.Module):
             taps = min(signal.shape[1], self.reverb_length)
             kernel = impulse.reshape(1, self.reverb_length)[:, :taps]
             signal = torch.ops.ddsp_b200.fftconv_fwd(signal.squeeze(-1), kernel, False)[0].unsqueeze(-1)
+        if self.streaming_reverb:
+            impulse = torch.ops.ddsp_b200.reverb_impulse_fwd(self.reverb_noise, self.reverb_decay, self.reverb_wet,
+                                                             self.reverb_t)
+            history = self.reverb_history.expand(signal.shape[0], self.reverb_length - 1).contiguous()
+            wet, history = torch.ops.ddsp_b200.conv_stream_fwd(signal.squeeze(-1), impulse, history)
+            self.reverb_history.copy_(history[:1])
+            signal = wet.unsqueeze(-1)
         return signal
 
     @torch.jit.export
     def reset(self):
-        """Forget the streaming state (GRU cache and oscillator phase)."""
+        """Forget the streaming state (GRU cache, oscillator phase and, when streamed, the reverb's input)."""
         self.cache_gru.zero_()
         self.phase.zero_()
+        if self.streaming_reverb:
+            self.reverb_history.zero_()
 
 
 def export_torchscript(model: DDSPDecoder, path: str, mean_loudness: float = 0.0, std_loudness: float = 1.0,
-                       realtime: bool = True, device_noise: bool = True) -> torch.jit.ScriptModule:
-    """export.py:55-65: script the wrapper and save it to ``path`` (a ``.ts`` file)."""
-    wrapper = ScriptDDSP(model.eval(), mean_loudness, std_loudness, realtime, device_noise).eval()
+                       realtime: bool = True, device_noise: bool = True,
+                       streaming_reverb: bool = False) -> torch.jit.ScriptModule:
+    """export.py:55-65: script the wrapper and save it to ``path`` (a ``.ts`` file).  ``streaming_reverb``
+    (realtime exports of a model with ``has_reverb`` only): play the trained reverb, its tail carried across calls."""
+    wrapper = ScriptDDSP(model.eval(), mean_loudness, std_loudness, realtime, device_noise, streaming_reverb).eval()
     scripted = torch.jit.script(wrapper)
     torch.jit.save(scripted, path)
     return scripted

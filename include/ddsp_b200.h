@@ -218,6 +218,19 @@ int ddsp_b200_reverb_impulse_bwd(const float *d_impulse, int Lvalid, const float
                                  const float *decay, const float *wet, const float *t,
                                  float *d_noise, float *d_decay, float *d_wet, int L, void *scratch, void *stream);
 
+/* ---- a10s  streaming reverb: Reverb.forward buffer by buffer     (ddsp/models/modules.py:28-35) ------
+ * modules.py:28-35 convolves one whole signal and crops the impulse to its length; played in buffers, the tail
+ * of each buffer is lost.  Here the previous L-1 input samples of each voice are carried by the caller:
+ *   u = [history | x] (B, L-1+N, oldest first);  y[b,n] = sum_{k<L} h[k] * u[b, L-1+n-k];
+ *   history_out[b] = the last L-1 samples of u[b]  (a separate buffer from history: both are read and written by
+ *   the same launch).  Zeros in history = silence before the first call.
+ * x[B,N], h[L] (one impulse for all voices), history / history_out [B,L-1] (may be NULL when L == 1), y[B,N].
+ * Direct form on the CUDA cores, B*N*L FMA (1 x 1024 x 48000 = 49 M per buffer); deterministic, no atomics.
+ * scratch: ddsp_b200_conv_stream_scratch(B, N, L) floats (the taps' chunk sums; 0 = none needed, may be NULL). */
+int64_t ddsp_b200_conv_stream_scratch(int B, int64_t N, int L);
+int ddsp_b200_conv_stream_fwd(const float *x, const float *h, const float *history, float *y, float *history_out,
+                              int B, int64_t N, int L, float *scratch, void *stream);
+
 /* ---- a11  multiscale_fft, one scale                           (ddsp/core.py:27-41) --------- */
 /* signal[B,N] -> mag[B, n_fft/2+1, frames], frames = 1 + N/hop (centred, reflect padded, periodic
  * Hann, normalised).  window[n_fft] is the float32 torch.hann_window(n_fft) the reference builds on

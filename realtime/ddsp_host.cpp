@@ -6,6 +6,8 @@
 // (ddsp_model.cpp:17), and the device is CUDA (ddsp_model.h:6).  No Pd dependency: `main` streams
 // synthetic 1024-sample buffers the way ddsp_tilde.cpp:81-92 does (a fresh std::thread per buffer) and
 // prints a checksum and the per-buffer latency, so the path can be exercised from a test.
+// All streaming state (GRU cache, oscillator phase and, in a streaming_reverb export, the reverb's history) lives
+// in the module's buffers: the same host plays a dry export and one that convolves its own reverb.
 //
 //   ddsp_host <libddsp_b200_torch.so> <model.ts> [buffers=8] [buffer_size=1024]
 #include <torch/script.h>
