@@ -27,7 +27,7 @@ __all__ = [
     "safe_log", "mean_std_loudness", "multiscale_fft", "resample", "upsample", "remove_above_nyquist",
     "scale_function", "extract_loudness", "extract_pitch", "mlp", "gru", "harmonic_synth",
     "amp_to_impulse_response", "fft_convolve",
-    "harmonic_synth_frames", "filtered_noise", "multiscale_spectral_loss", "convolve_stream",
+    "harmonic_synth_frames", "filtered_noise", "multiscale_spectral_loss", "convolve_stream", "extract_features",
 ]
 
 
@@ -89,8 +89,30 @@ def scale_function(x):
     return _F.ScaleFunction.apply(x)
 
 
+def _feature_rows(signal, name: str):
+    if torch.is_grad_enabled() and signal.requires_grad:
+        raise RuntimeError(f"{name} has no backward: call it under torch.no_grad() or on a detached tensor")
+    if signal.dim() not in (1, 2):
+        raise ValueError(f"{name}: signal must be (N,) or (B, N), got {tuple(signal.shape)}")
+    return signal.unsqueeze(0) if signal.dim() == 1 else signal
+
+
+def _features(signal, sample_rate, block_size: int, n_fft: int, n_mfcc: int, mfcc: bool, name: str):
+    rows = _feature_rows(signal, name)
+    window, a_weight, mel, dct = _F.feature_tables(sample_rate, n_fft, n_mfcc, signal.device)
+    loud, coeffs = _F._ops.features_fwd(rows, window, a_weight, mel, dct, int(n_fft), int(block_size), mfcc)
+    if signal.dim() == 1:
+        return loud[0], (coeffs[0] if mfcc else coeffs)
+    return loud, coeffs
+
+
 def extract_loudness(signal, sample_rate, block_size, n_fft=2048):
-    """ddsp/core.py:81-97 (offline preprocessing, numpy + librosa; out of the hot path)."""
+    """ddsp/core.py:81-97: A-weighted loudness, mean over bins of log(|STFT| + 1e-7) + A_weighting, one value per
+    block.  A CUDA float32 tensor (N,) or (B, N) runs on the feature kernel (csrc/features.cu) and returns
+    (..., N // block_size); anything else takes the reference's numpy + librosa code (offline preprocessing)."""
+    if isinstance(signal, torch.Tensor) and signal.is_cuda and signal.dtype == torch.float32 and signal.dim() in (1, 2):
+        loud, _ = _features(signal, sample_rate, block_size, n_fft, 1, False, "extract_loudness")
+        return loud[..., :-1]
     import numpy as np
     import librosa as li
     spec = li.stft(signal, n_fft=n_fft, hop_length=block_size, win_length=n_fft, center=True)
@@ -302,6 +324,18 @@ def convolve_stream(signal, kernel, history: Optional[torch.Tensor] = None):
     if torch.is_grad_enabled() and any(t.requires_grad for t in (signal, kernel, history)):
         raise RuntimeError("convolve_stream has no backward: call it under torch.no_grad() or on detached tensors")
     return _F._ops.conv_stream_fwd(signal, kernel, history)
+
+
+def extract_features(signal, sample_rate, block_size, n_mfcc=30, n_fft=2048):
+    """Extension: the two signal-processing features of a dataset from one pass of the feature kernel over a CUDA
+    float32 signal (N,) or (B, N): -> (loudness (..., N // block_size) as ``extract_loudness``,
+    mfcc (..., 1 + N // block_size, n_mfcc) as ``librosa.feature.mfcc(y, sr, n_mfcc=n_mfcc, n_fft=n_fft,
+    hop_length=block_size)`` with its defaults: 128 Slaney mel bands, power_to_db with top_db = 80 per row,
+    DCT-II ortho; the layout of ``mfccs.npy``).  Forward only: an input that requires grad raises under grad mode."""
+    if not 1 <= int(n_mfcc) <= _F.N_MELS:
+        raise ValueError(f"extract_features: n_mfcc must be in 1..{_F.N_MELS}, got {n_mfcc}")
+    loud, mfcc = _features(signal, sample_rate, block_size, n_fft, int(n_mfcc), True, "extract_features")
+    return loud[..., :-1], mfcc
 
 
 def multiscale_spectral_loss(target, rec, scales: Sequence[int], overlap: float):

@@ -685,6 +685,38 @@ std::tuple<Tensor, Tensor> conv_stream_fwd(const Tensor &signal_, const Tensor &
     return {y, hist_out};
 }
 
+// ---------------------------------------------------------------------------------------- f1 dataset features
+// signal (B,N) -> (loudness (B,F), mfcc (B,F,n_mfcc) or an empty tensor when mfcc is false), F = 1 + N/hop.
+// a_weight (n_fft/2+1), mel_table (the compact band table of the C ABI), dct (128, n_mfcc): functions.feature_tables.
+std::tuple<Tensor, Tensor> features_fwd(const Tensor &signal_, const Tensor &window_, const Tensor &a_weight_,
+                                        const Tensor &mel_table_, const Tensor &dct_, int64_t n_fft, int64_t hop,
+                                        bool mfcc) {
+    Tensor sig = prep(signal_, "signal"), win = prep(window_, "window"), aw = prep(a_weight_, "a_weight");
+    Tensor mel = prep(mel_table_, "mel_table"), dct = prep(dct_, "dct");
+    TORCH_CHECK(sig.dim() == 2, "features: signal must be (B,N)");
+    TORCH_CHECK(win.numel() == n_fft && aw.numel() == n_fft / 2 + 1, "features: window (n_fft) and a_weight (n_fft/2+1) expected");
+    TORCH_CHECK(dct.dim() == 2 && dct.size(0) == 128, "features: dct must be (128, n_mfcc)");
+    TORCH_CHECK(mel.numel() >= 384, "features: mel_table is shorter than its header");
+    for (const Tensor *t : {&win, &aw, &mel, &dct})
+        TORCH_CHECK(t->device() == sig.device(), "features: tensors on different devices");
+    const int64_t B = sig.size(0), N = sig.size(1), n_mfcc = dct.size(1);
+    TORCH_CHECK(B <= INT32_MAX && n_fft <= 4096 && hop >= 1 && hop <= INT32_MAX, "features: unsupported sizes");
+    c10::cuda::CUDAGuard guard(sig.device());
+    const int64_t ns = ddsp_b200_features_scratch((int)B, N, (int)n_fft, (int)hop, (int)n_mfcc);
+    TORCH_CHECK(ns > 0, "features: unsupported sizes (B ", B, ", N ", N, ", n_fft ", n_fft, ", hop ", hop,
+                ", n_mfcc ", n_mfcc, ")");
+    const int64_t F = 1 + N / hop;
+    Tensor loud = at::empty({B, F}, sig.options());
+    Tensor out = at::empty({mfcc ? B : 0, F, n_mfcc}, sig.options());
+    Tensor scratch = mfcc ? at::empty({ns}, sig.options()) : Tensor();
+    Tensor stw = stage_twiddle_table(sig.device(), n_fft);
+    check(ddsp_b200_features_fwd(fp(sig), fp(win), fp(stw), fp(aw), fp(mel), fp(dct), fpm(loud),
+                                 mfcc ? fpm(out) : nullptr, mfcc ? fpm(scratch) : nullptr, (int)B, N, (int)n_fft,
+                                 (int)hop, (int)n_mfcc, cur_stream()),
+          "features_fwd");
+    return {loud, out};
+}
+
 // ---------------------------------------------------------------------------------------- a11, a12
 int64_t pow2_ge(int64_t v) {
     int64_t p = 1;
@@ -1003,6 +1035,7 @@ TORCH_LIBRARY(ddsp_b200, m) {
     m.def("reverb_impulse_fwd(Tensor noise, Tensor decay, Tensor wet, Tensor t) -> Tensor");
     m.def("reverb_impulse_bwd(Tensor d_impulse, Tensor noise, Tensor decay, Tensor wet, Tensor t) -> (Tensor, Tensor, Tensor)");
     m.def("conv_stream_fwd(Tensor signal, Tensor kernel, Tensor history) -> (Tensor, Tensor)");
+    m.def("features_fwd(Tensor signal, Tensor window, Tensor a_weight, Tensor mel_table, Tensor dct, int n_fft, int hop, bool mfcc) -> (Tensor, Tensor)");
     m.def("stft_mag_fwd(Tensor signal, Tensor window, int n_fft, int hop) -> Tensor");
     m.def("stft_mag_bwd(Tensor signal, Tensor d_mag, Tensor window, int n_fft, int hop) -> Tensor");
     m.def("mss_loss_fwd(Tensor target, Tensor rec, int[] scales, float overlap, Tensor windows, bool need_grad) -> (Tensor, Tensor)");
@@ -1039,6 +1072,7 @@ TORCH_LIBRARY_IMPL(ddsp_b200, CUDA, m) {
     m.impl("reverb_impulse_fwd", reverb_impulse_fwd);
     m.impl("reverb_impulse_bwd", reverb_impulse_bwd);
     m.impl("conv_stream_fwd", conv_stream_fwd);
+    m.impl("features_fwd", features_fwd);
     m.impl("stft_mag_fwd", stft_mag_fwd);
     m.impl("stft_mag_bwd", stft_mag_bwd);
     m.impl("mss_loss_fwd", mss_loss_fwd);

@@ -8,6 +8,7 @@ from __future__ import annotations
 
 from typing import List, Optional, Sequence
 
+import numpy as np
 import torch
 from torch.autograd.function import once_differentiable
 
@@ -40,6 +41,91 @@ def hann_windows_like_reference(scales: Sequence[int], device) -> torch.Tensor:
         w = torch.cat([hann_window_like_reference(s, device) for s in key[0]])
         _WINDOW_SETS[key] = w
     return w
+
+
+# ---- constant tables of the feature extractor (csrc/features.cu), built in float64 on the host ----------------------
+N_MELS = 128
+
+
+def a_weighting_db(freqs) -> np.ndarray:
+    """librosa's ``A_weighting`` (min_db = -80) in dB at ``freqs`` Hz, float64."""
+    f2 = np.asarray(freqs, np.float64) ** 2
+    c = np.array([12194.217, 20.598997, 107.65265, 737.86223]) ** 2
+    with np.errstate(divide="ignore"):
+        a = 2.0 + 20.0 * (np.log10(c[0]) + 2 * np.log10(f2) - np.log10(f2 + c[0]) - np.log10(f2 + c[1])
+                          - 0.5 * np.log10(f2 + c[2]) - 0.5 * np.log10(f2 + c[3]))
+    return np.maximum(-80.0, a)
+
+
+def _hz_to_mel(f):
+    """Slaney mel scale (librosa ``htk=False``): linear below 1 kHz, logarithmic above."""
+    f = np.asarray(f, np.float64)
+    logstep = np.log(6.4) / 27.0
+    return np.where(f >= 1000.0, 15.0 + np.log(np.maximum(f, 1e-300) / 1000.0) / logstep, f / (200.0 / 3))
+
+
+def _mel_to_hz(m):
+    m = np.asarray(m, np.float64)
+    logstep = np.log(6.4) / 27.0
+    return np.where(m >= 15.0, 1000.0 * np.exp(logstep * (m - 15.0)), m * (200.0 / 3))
+
+
+def mel_filterbank(sample_rate: float, n_fft: int, n_mels: int = N_MELS) -> np.ndarray:
+    """``librosa.filters.mel(sr, n_fft, n_mels, fmin=0, fmax=sr/2, htk=False, norm="slaney")``: (n_mels, n_fft/2+1)
+    float64 triangles on the Slaney mel scale, each scaled to unit area (2 / its width in Hz)."""
+    fft_freqs = np.linspace(0.0, sample_rate / 2, 1 + n_fft // 2)
+    mel_f = _mel_to_hz(np.linspace(_hz_to_mel(0.0), _hz_to_mel(sample_rate / 2), n_mels + 2))
+    fdiff = np.diff(mel_f)
+    ramps = mel_f[:, None] - fft_freqs[None, :]
+    lower = -ramps[:-2] / fdiff[:-1, None]
+    upper = ramps[2:] / fdiff[1:, None]
+    weights = np.maximum(0.0, np.minimum(lower, upper))
+    return weights * (2.0 / (mel_f[2:] - mel_f[:-2]))[:, None]
+
+
+def mel_band_table(weights: np.ndarray) -> np.ndarray:
+    """The compact band table the kernel reads: first bin, bin count and weight offset of each band (as floats, exact
+    below 2^24), then every band's nonzero run of weights back to back.  float32."""
+    n_mels = weights.shape[0]
+    first, count, offset, runs, pos = [], [], [], [], 0
+    for row in weights:
+        nz = np.nonzero(row)[0]
+        lo, hi = (int(nz[0]), int(nz[-1]) + 1) if nz.size else (0, 0)
+        first.append(lo)
+        count.append(hi - lo)
+        offset.append(pos)
+        runs.append(row[lo:hi])
+        pos += hi - lo
+    head = np.array([first, count, offset], np.float64).reshape(3 * n_mels)
+    return np.concatenate([head] + runs).astype(np.float32)
+
+
+def dct_matrix(n_mfcc: int, n_mels: int = N_MELS) -> np.ndarray:
+    """DCT-II with ``norm="ortho"``, the first n_mfcc rows: (n_mfcc, n_mels) float64."""
+    i = np.arange(n_mfcc, dtype=np.float64)[:, None]
+    j = np.arange(n_mels, dtype=np.float64)[None, :]
+    d = np.cos(np.pi * i * (2 * j + 1) / (2 * n_mels)) * np.sqrt(2.0 / n_mels)
+    d[0] *= np.sqrt(0.5)
+    return d
+
+
+_FEATURE_TABLES = {}
+
+
+def feature_tables(sample_rate: float, n_fft: int, n_mfcc: int, device):
+    """(window, a_weight, mel_table, dct (128, n_mfcc)) for ``features_fwd``, built once per
+    (sample_rate, n_fft, n_mfcc, device)."""
+    key = (float(sample_rate), int(n_fft), int(n_mfcc), str(device))
+    tabs = _FEATURE_TABLES.get(key)
+    if tabs is None:
+        sr, n_fft = key[0], key[1]
+        freqs = np.arange(n_fft // 2 + 1, dtype=np.float64) * sr / n_fft
+        tabs = (hann_window_like_reference(n_fft, device),
+                torch.from_numpy(a_weighting_db(freqs).astype(np.float32)).to(device),
+                torch.from_numpy(mel_band_table(mel_filterbank(sr, n_fft))).to(device),
+                torch.from_numpy(np.ascontiguousarray(dct_matrix(key[2]).T).astype(np.float32)).to(device))
+        _FEATURE_TABLES[key] = tabs
+    return tabs
 
 
 class ScaleFunction(torch.autograd.Function):

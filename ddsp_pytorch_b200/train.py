@@ -6,8 +6,10 @@ The reference's ``train.py`` is a single-device, module-level script around a Li
 
 * data: the reference's on-disk format (``signals.npy``, ``pitchs.npy``, ``loudness.npy``, ``mfccs.npy`` in one
   directory, ``data.py:13-16``), memory-mapped, batches with the reference's keys (``sig``, ``pitch``,
-  ``loudness``, ``mfcc``; the last MFCC frame dropped as at ``data.py:25``); ``write_synthetic_dataset`` makes a
-  dataset of that format without the offline feature extractors (librosa / CREPE are not part of this repo);
+  ``loudness``, ``mfcc``; the last MFCC frame dropped as at ``data.py:25``); ``tools/extract_features.py`` writes a
+  dataset's ``loudness.npy`` and ``mfccs.npy`` from its ``signals.npy`` on the GPU (``core.extract_features``; pitch
+  needs CREPE, which is not part of this repo); ``write_synthetic_dataset`` makes a dataset of that format with
+  synthetic features;
 * every rank takes a disjoint, equal slice of each global batch (``distributed.shard_range``), batches are
   staged through pinned host memory one step ahead on a copy stream;
 * step: loudness standardised with the training-set statistics (``train.py:86``), model forward, fused
@@ -68,7 +70,10 @@ class NpyDataset(torch.utils.data.Dataset):
 def write_synthetic_dataset(out_dir, n_examples: int, sample_rate: int = 16000, block_size: int = 160,
                             seconds: float = 4.0, n_mfcc: int = 30, seed: int = 0) -> Path:
     """A dataset in the reference's format (``preprocess.py:77-88`` writes the same four arrays) made of
-    harmonic tones with a slow vibrato and a loudness envelope, so that a model can actually fit it."""
+    harmonic tones with a slow vibrato and a loudness envelope, so that a model can actually fit it.  The pitch and
+    loudness arrays are the synthesis controls; ``mfccs.npy`` is standard-normal noise.  Run
+    ``tools/extract_features.py --overwrite`` on the directory to replace loudness and MFCCs by the features of the
+    signals themselves."""
     out_dir = Path(out_dir)
     out_dir.mkdir(parents=True, exist_ok=True)
     rng = np.random.default_rng(seed)

@@ -231,6 +231,23 @@ int64_t ddsp_b200_conv_stream_scratch(int B, int64_t N, int L);
 int ddsp_b200_conv_stream_fwd(const float *x, const float *h, const float *history, float *y, float *history_out,
                               int B, int64_t N, int L, float *scratch, void *stream);
 
+/* ---- f1  dataset features: A-weighted loudness and MFCCs  (ddsp/core.py:81-97, librosa.feature.mfcc defaults) --
+ * signal[B,N] -> F = 1 + N/hop frames of the unnormalised STFT (reflect padding of n_fft/2 on each side, periodic
+ * Hann window[n_fft]), bins k = 0 .. n_fft/2.
+ *   loudness[B,F]  = mean over k of ln(|X[k]| + 1e-7) + a_weight[k]           (a_weight: A-weighting in dB, n_fft/2+1)
+ *   mfcc[B,F,n_mfcc]: P = |X|^2, mel = 128 Slaney bands of P, dB = 10 log10(max(1e-10, mel)) clamped per row to
+ *                    its maximum - 80, then dct[128][n_mfcc] (the DCT-II ortho matrix, transposed) applied to dB.
+ * mel_table: floats [0,128) first bin, [128,256) bin count, [256,384) offset of the band's weights past the
+ * header, then the weights back to back.  stage_twiddle: ddsp_b200_fft_stage_twiddles(n_fft).
+ * loudness or mfcc may be NULL (not both); without mfcc, mel_table / dct / scratch may be NULL and one launch runs.
+ * scratch: ddsp_b200_features_scratch(...) floats.  n_fft a power of two in 256..4096, 1 <= hop <= 2^30,
+ * n_fft/2 < N < 2^30, 1 <= n_mfcc <= 128, 1 <= B <= 65535, else DDSP_B200_EINVAL (both functions).
+ * Deterministic: sums in a fixed order, a row's output does not depend on the batch it is computed in.         */
+int64_t ddsp_b200_features_scratch(int B, int64_t N, int n_fft, int hop, int n_mfcc);
+int ddsp_b200_features_fwd(const float *signal, const float *window, const float *stage_twiddle, const float *a_weight,
+                           const float *mel_table, const float *dct, float *loudness, float *mfcc, float *scratch,
+                           int B, int64_t N, int n_fft, int hop, int n_mfcc, void *stream);
+
 /* ---- a11  multiscale_fft, one scale                           (ddsp/core.py:27-41) --------- */
 /* signal[B,N] -> mag[B, n_fft/2+1, frames], frames = 1 + N/hop (centred, reflect padded, periodic
  * Hann, normalised).  window[n_fft] is the float32 torch.hann_window(n_fft) the reference builds on
