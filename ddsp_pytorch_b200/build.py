@@ -23,7 +23,7 @@ INCLUDE = os.path.join(ROOT, "include")
 LIB_CORE = os.path.join(PKG, "libddsp_b200.so")
 LIB_TORCH = os.path.join(PKG, "libddsp_b200_torch.so")
 
-CU_SOURCES = ["controls.cu", "harmonic.cu", "noise.cu", "stft.cu", "mss_fused.cu", "fftconv.cu", "conv_stream.cu", "features.cu", "gru.cu", "gemm3x.cu", "layernorm.cu"]
+CU_SOURCES = ["controls.cu", "harmonic.cu", "noise.cu", "stft.cu", "mss_fused.cu", "fftconv.cu", "conv_stream.cu", "features.cu", "pitch.cu", "gru.cu", "gemm3x.cu", "layernorm.cu"]
 CU_HEADERS = ["common.cuh", "fft.cuh", "regfft.cuh", "pfft.cuh"]
 ARCH = ["-gencode", "arch=compute_100a,code=sm_100a"]
 

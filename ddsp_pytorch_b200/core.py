@@ -28,6 +28,7 @@ __all__ = [
     "scale_function", "extract_loudness", "extract_pitch", "mlp", "gru", "harmonic_synth",
     "amp_to_impulse_response", "fft_convolve",
     "harmonic_synth_frames", "filtered_noise", "multiscale_spectral_loss", "convolve_stream", "extract_features",
+    "extract_pitch_yin",
 ]
 
 
@@ -336,6 +337,43 @@ def extract_features(signal, sample_rate, block_size, n_mfcc=30, n_fft=2048):
         raise ValueError(f"extract_features: n_mfcc must be in 1..{_F.N_MELS}, got {n_mfcc}")
     loud, mfcc = _features(signal, sample_rate, block_size, n_fft, int(n_mfcc), True, "extract_features")
     return loud[..., :-1], mfcc
+
+
+def _yin_periods(sample_rate, fmin, fmax, frame_length: int = 2048):
+    """The lag range of ``extract_pitch_yin``, in samples, as librosa.yin derives it:
+    (max(floor(sr / fmax), 1), min(ceil(sr / fmin), frame_length - frame_length // 2 - 1))."""
+    sr, fmin, fmax = float(sample_rate), float(fmin), float(fmax)
+    if not fmin > 0.0:
+        raise ValueError(f"extract_pitch_yin: fmin must be > 0, got {fmin}")
+    if not fmin < fmax:
+        raise ValueError(f"extract_pitch_yin: fmin ({fmin}) must be below fmax ({fmax})")
+    if fmax > sr / 2:
+        raise ValueError(f"extract_pitch_yin: fmax ({fmax}) is above the Nyquist frequency ({sr / 2})")
+    L = int(frame_length)
+    min_period = max(int(math.floor(sr / fmax)), 1)
+    max_period = min(int(math.ceil(sr / fmin)), L - L // 2 - 1)
+    if max_period < min_period + 2:
+        raise ValueError(f"extract_pitch_yin: the lag range {min_period}..{max_period} of fmin {fmin}, fmax {fmax} at "
+                         f"frame_length {L} is empty (it needs three lags at least)")
+    return min_period, max_period
+
+
+def extract_pitch_yin(signal, sample_rate, block_size, fmin, fmax, frame_length=2048, threshold=0.1):
+    """Extension: the pitch of a CUDA float32 signal (N,) or (B, N) by YIN (csrc/pitch.cu), one value per block like
+    ``extract_pitch`` and ``extract_loudness``: -> (f0 (..., N // block_size) in Hz, aperiodicity (..., N // block_size)).
+    librosa.yin's definition with the frames of ``extract_loudness`` (reflect padding of frame_length/2, window
+    frame_length/2): the first trough of the cumulative mean normalised difference below ``threshold``, else its
+    global minimum, refined by a parabola.  The aperiodicity is the normalised difference at the chosen lag (YIN's
+    voicing measure: small for periodic frames).  No smoothing: unvoiced frames take the global minimum, and an
+    all-zero frame gives f0 = sample_rate / floor(sample_rate / fmax) with aperiodicity 0, as in librosa.
+    Forward only: an input that requires grad raises under grad mode."""
+    rows = _feature_rows(signal, "extract_pitch_yin")
+    min_period, max_period = _yin_periods(sample_rate, fmin, fmax, frame_length)
+    f0, ap = _F._ops.pitch_yin_fwd(rows, int(frame_length), int(block_size), min_period, max_period,
+                                   float(sample_rate), float(threshold))
+    if signal.dim() == 1:
+        return f0[0], ap[0]
+    return f0, ap
 
 
 def multiscale_spectral_loss(target, rec, scales: Sequence[int], overlap: float):

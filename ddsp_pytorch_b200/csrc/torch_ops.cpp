@@ -717,6 +717,28 @@ std::tuple<Tensor, Tensor> features_fwd(const Tensor &signal_, const Tensor &win
     return {loud, out};
 }
 
+// ---------------------------------------------------------------------------------------- f1 dataset pitch (YIN)
+// signal (B,N) -> (f0 (B,F), aperiodicity (B,F)), F = N/hop; the periods come from core.extract_pitch_yin.
+std::tuple<Tensor, Tensor> pitch_yin_fwd(const Tensor &signal_, int64_t frame_length, int64_t hop, int64_t min_period,
+                                         int64_t max_period, double sample_rate, double threshold) {
+    Tensor sig = prep(signal_, "signal");
+    TORCH_CHECK(sig.dim() == 2, "pitch_yin: signal must be (B,N)");
+    const int64_t B = sig.size(0), N = sig.size(1);
+    TORCH_CHECK(B >= 1 && B <= 65535 && frame_length >= 256 && frame_length <= 4096 &&
+                    (frame_length & (frame_length - 1)) == 0 && hop >= 1 && hop <= INT32_MAX && min_period >= 1 &&
+                    max_period <= frame_length / 2 - 1 && max_period >= min_period + 2,
+                "pitch_yin: unsupported sizes (B ", B, ", frame_length ", frame_length, ", hop ", hop, ", periods ",
+                min_period, "..", max_period, ")");
+    c10::cuda::CUDAGuard guard(sig.device());
+    const int64_t F = N / hop;
+    Tensor f0 = at::empty({B, F}, sig.options()), ap = at::empty({B, F}, sig.options());
+    Tensor stw = stage_twiddle_table(sig.device(), frame_length);
+    check(ddsp_b200_pitch_yin_fwd(fp(sig), fp(stw), fpm(f0), fpm(ap), (int)B, N, (int)frame_length, (int)hop,
+                                  (int)min_period, (int)max_period, (float)sample_rate, (float)threshold, cur_stream()),
+          "pitch_yin_fwd");
+    return {f0, ap};
+}
+
 // ---------------------------------------------------------------------------------------- a11, a12
 int64_t pow2_ge(int64_t v) {
     int64_t p = 1;
@@ -1036,6 +1058,7 @@ TORCH_LIBRARY(ddsp_b200, m) {
     m.def("reverb_impulse_bwd(Tensor d_impulse, Tensor noise, Tensor decay, Tensor wet, Tensor t) -> (Tensor, Tensor, Tensor)");
     m.def("conv_stream_fwd(Tensor signal, Tensor kernel, Tensor history) -> (Tensor, Tensor)");
     m.def("features_fwd(Tensor signal, Tensor window, Tensor a_weight, Tensor mel_table, Tensor dct, int n_fft, int hop, bool mfcc) -> (Tensor, Tensor)");
+    m.def("pitch_yin_fwd(Tensor signal, int frame_length, int hop, int min_period, int max_period, float sample_rate, float threshold) -> (Tensor, Tensor)");
     m.def("stft_mag_fwd(Tensor signal, Tensor window, int n_fft, int hop) -> Tensor");
     m.def("stft_mag_bwd(Tensor signal, Tensor d_mag, Tensor window, int n_fft, int hop) -> Tensor");
     m.def("mss_loss_fwd(Tensor target, Tensor rec, int[] scales, float overlap, Tensor windows, bool need_grad) -> (Tensor, Tensor)");
@@ -1073,6 +1096,7 @@ TORCH_LIBRARY_IMPL(ddsp_b200, CUDA, m) {
     m.impl("reverb_impulse_bwd", reverb_impulse_bwd);
     m.impl("conv_stream_fwd", conv_stream_fwd);
     m.impl("features_fwd", features_fwd);
+    m.impl("pitch_yin_fwd", pitch_yin_fwd);
     m.impl("stft_mag_fwd", stft_mag_fwd);
     m.impl("stft_mag_bwd", stft_mag_bwd);
     m.impl("mss_loss_fwd", mss_loss_fwd);

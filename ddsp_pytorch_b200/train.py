@@ -7,8 +7,9 @@ The reference's ``train.py`` is a single-device, module-level script around a Li
 * data: the reference's on-disk format (``signals.npy``, ``pitchs.npy``, ``loudness.npy``, ``mfccs.npy`` in one
   directory, ``data.py:13-16``), memory-mapped, batches with the reference's keys (``sig``, ``pitch``,
   ``loudness``, ``mfcc``; the last MFCC frame dropped as at ``data.py:25``); ``tools/extract_features.py`` writes a
-  dataset's ``loudness.npy`` and ``mfccs.npy`` from its ``signals.npy`` on the GPU (``core.extract_features``; pitch
-  needs CREPE, which is not part of this repo); ``write_synthetic_dataset`` makes a dataset of that format with
+  dataset's ``loudness.npy`` and ``mfccs.npy`` from its ``signals.npy`` on the GPU (``core.extract_features``), and
+  with ``--pitch`` its ``pitchs.npy`` by YIN (``core.extract_pitch_yin``; the reference used CREPE, which is not part of
+  this repo), so recordings alone make a dataset; ``write_synthetic_dataset`` makes a dataset of that format with
   synthetic features;
 * every rank takes a disjoint, equal slice of each global batch (``distributed.shard_range``), batches are
   staged through pinned host memory one step ahead on a copy stream;

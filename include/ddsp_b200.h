@@ -248,6 +248,24 @@ int ddsp_b200_features_fwd(const float *signal, const float *window, const float
                            const float *mel_table, const float *dct, float *loudness, float *mfcc, float *scratch,
                            int B, int64_t N, int n_fft, int hop, int n_mfcc, void *stream);
 
+/* ---- f1  dataset pitch: YIN  (replaces ddsp/core.py:100-119, CREPE; librosa.yin's definition) --------------------
+ * signal[B,N] -> N/hop frames x of L = frame_length samples (reflect padding of L/2 on each side, frame f starts at
+ * f*hop of the padded signal: the frames of the loudness), W = L/2.  For tau = 0 .. max_period:
+ *   d(tau) = max(0, sum_{j=1..W} (x[j] - x[j+tau])^2)      (computed as E(0) + E(tau) - 2 acf(tau) by one FFT pair)
+ *   y(tau) = d(tau) / (sum_{k=1..tau} d(k) / tau + FLT_MIN),   tau in [min_period, max_period]
+ * lag = the first trough of y (y(tau) < y(tau-1) and y(tau) <= y(tau+1); at min_period y < y(tau+1); never at
+ * max_period) with y < threshold, else the first global minimum of y.  Parabolic shift s = -b/a through y(lag-1),
+ * y(lag), y(lag+1) (a = y+ + y- - 2y, b = (y+ - y-)/2; 0 at either end of the range or when |b| >= |a|).
+ *   f0[B, N/hop] = sample_rate / (lag + s)          aperiodicity[B, N/hop] = y(lag)
+ * An all-zero frame has y == 0 and no trough: f0 = sample_rate / min_period, aperiodicity 0.
+ * stage_twiddle: ddsp_b200_fft_stage_twiddles(frame_length).  DDSP_B200_EINVAL before any launch unless
+ * 1 <= B <= 65535, L/2 < N < 2^30, L a power of two in 256..4096, hop >= 1, min_period >= 1,
+ * min_period + 2 <= max_period <= L - W - 1, threshold finite, and no pointer NULL.
+ * Deterministic: fixed-order sums, no atomics; a row's output does not depend on the batch it is computed in.    */
+int ddsp_b200_pitch_yin_fwd(const float *signal, const float *stage_twiddle, float *f0, float *aperiodicity, int B,
+                            int64_t N, int frame_length, int hop, int min_period, int max_period, float sample_rate,
+                            float threshold, void *stream);
+
 /* ---- a11  multiscale_fft, one scale                           (ddsp/core.py:27-41) --------- */
 /* signal[B,N] -> mag[B, n_fft/2+1, frames], frames = 1 + N/hop (centred, reflect padded, periodic
  * Hann, normalised).  window[n_fft] is the float32 torch.hann_window(n_fft) the reference builds on
