@@ -24,6 +24,42 @@ static inline int ddsp_launch_status() {
 
 static inline int64_t ddsp_ceil_div(int64_t a, int64_t b) { return (a + b - 1) / b; }
 
+// Launch as the programmatic dependent of the kernel launched before it on `st`: dispatched once every CTA of that
+// kernel has run griddepcontrol.launch_dependents (or exited), not when it ends.  The kernel must read nothing the
+// earlier one writes (it never calls griddepcontrol.wait).
+template <typename... P, typename... A>
+int ddsp_launch_programmatic(void (*kernel)(P...), dim3 grid, dim3 block, size_t smem, cudaStream_t st, A &&...args) {
+    cudaLaunchConfig_t cfg = {};
+    cfg.gridDim = grid;
+    cfg.blockDim = block;
+    cfg.dynamicSmemBytes = smem;
+    cfg.stream = st;
+    cudaLaunchAttribute attr;
+    attr.id = cudaLaunchAttributeProgrammaticStreamSerialization;
+    attr.val.programmaticStreamSerializationAllowed = 1;
+    cfg.attrs = &attr;
+    cfg.numAttrs = 1;
+    const cudaError_t e = cudaLaunchKernelEx(&cfg, kernel, static_cast<A &&>(args)...);
+    if (e != cudaSuccess) {
+        cudaGetLastError();
+        return (int)e;
+    }
+    return ddsp_launch_status();
+}
+
+// The oscillator bank's half of the synth pair (harmonic.cu), launched as the programmatic dependent of the filtered
+// noise by ddsp_b200_synth_pair_fwd / _bwd (noise.cu).  Same arguments and results as
+// ddsp_b200_harmonic_frames_raw_scan_fwd / ddsp_b200_harmonic_frames_raw_bwd.
+bool ddsp_pair_bank_supported(int T, int H, int block_size);
+int ddsp_pair_bank_fwd(const float *amp_raw, int64_t amp_stride, const float *dist_raw, int64_t dist_stride,
+                       const float *f0, const double *phase0, uint64_t *phi, uint64_t *delta, double *phase_end,
+                       float *amps, float *weights, float *audio, int B, int T, int H, int block_size,
+                       double sample_rate, cudaStream_t st);
+int ddsp_pair_bank_bwd(const float *g_audio, const float *amp_raw, int64_t amp_stride, const float *dist_raw,
+                       int64_t dist_stride, const float *f0, const uint64_t *phi, const uint64_t *delta,
+                       float *d_amp_raw, int64_t d_amp_stride, float *d_dist_raw, int64_t d_dist_stride, int B, int T,
+                       int H, int block_size, float sample_rate, cudaStream_t st);
+
 // ---------------------------------------------------------------------------------------------
 // Phase arithmetic.  Phases are kept in TURNS as Q0.64 unsigned fixed point: wrap-around of the
 // 64-bit integer is exactly "mod 1 turn", so k*phase for harmonic k is exact however long the

@@ -680,8 +680,10 @@ static int frames_per_cta(int bs, int T, int sweep, int cap) {
 }
 
 // shared by the two forward entry points; rc = nullptr: weights are read, else computed in the prologue
+// programmatic: launched as the programmatic dependent of the kernel before it on `st` (the synth pair)
 static int launch_frames_fwd(const float *weights, const RawControls *rc, const uint64_t *phi, const uint64_t *delta,
-                             float *audio, int B, int T, int H, int block_size, cudaStream_t st) {
+                             float *audio, int B, int T, int H, int block_size, cudaStream_t st,
+                             bool programmatic = false) {
     const int bs = block_size;
     const int bsp = (bs + 3) & ~3;                                      // frame length in whole groups of 4 samples
     const int Hp = (H + 3) & ~3;
@@ -704,6 +706,9 @@ static int launch_frames_fwd(const float *weights, const RawControls *rc, const 
     if (threads > kFwdMaxThreads) threads = kFwdMaxThreads;
     auto kernel = rc ? harmonic_frames_fwd_x2_kernel<true> : harmonic_frames_fwd_x2_kernel<false>;
     if (smem > 48 * 1024) cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    if (programmatic)
+        return ddsp_launch_programmatic(kernel, grid, dim3(threads), smem, st, weights, phi, delta, audio, T, H, Hp, bs,
+                                        fr, rc ? *rc : RawControls{});
     kernel<<<grid, threads, smem, st>>>(weights, phi, delta, audio, T, H, Hp, bs, fr, rc ? *rc : RawControls{});
     return ddsp_launch_status();
 }
@@ -761,8 +766,30 @@ extern "C" int ddsp_b200_harmonic_frames_raw_scan_fwd(const float *amp_raw, int6
     return launch_frames_fwd(nullptr, &rc, phi, delta, audio, B, T, H, block_size, (cudaStream_t)stream);
 }
 
+// The synth pair takes the bank with the scan inside the launch only: a separate scan launch would be the noise
+// kernel's dependent instead, and the bank would wait for the noise to finish.
+bool ddsp_pair_bank_supported(int T, int H, int block_size) {
+    if (T < 1 || !ddsp_b200_harmonic_frames_raw_supported(H, block_size)) return false;
+    const int fr = frames_per_cta(block_size, T, kFwdThreads * 4, 32);
+    return (T + fr - 1) / fr <= 64;
+}
+
+int ddsp_pair_bank_fwd(const float *amp_raw, int64_t amp_stride, const float *dist_raw, int64_t dist_stride,
+                       const float *f0, const double *phase0, uint64_t *phi, uint64_t *delta, double *phase_end,
+                       float *amps, float *weights, float *audio, int B, int T, int H, int block_size,
+                       double sample_rate, cudaStream_t st) {
+    DDSP_REQUIRE(amp_raw && dist_raw && f0 && phi && delta && amps && weights && audio);
+    DDSP_REQUIRE(B > 0 && B <= 65535 && T > 0 && H > 0 && block_size > 0 && amp_stride >= 1 && dist_stride >= H);
+    DDSP_REQUIRE(sample_rate > 0);
+    if (!ddsp_pair_bank_supported(T, H, block_size)) return DDSP_B200_EUNSUPPORTED;
+    RawControls rc{amp_raw, dist_raw, f0, amp_stride, dist_stride, (float)sample_rate * 0.5f, amps, weights,
+                   1, block_size, make_phase_k(1.0 / sample_rate), phase0, phase_end, phi, delta};
+    return launch_frames_fwd(nullptr, &rc, phi, delta, audio, B, T, H, block_size, st, true);
+}
+
 static int launch_frames_bwd(const float *g_audio, const uint64_t *phi, const uint64_t *delta, float *d_weights,
-                             const RawControlsGrad *rc, int B, int T, int H, int block_size, cudaStream_t st) {
+                             const RawControlsGrad *rc, int B, int T, int H, int block_size, cudaStream_t st,
+                             bool programmatic = false) {
     const int bs = block_size;
     const int nchunk = (bs + kChunk - 1) / kChunk;
     const int clen = (((bs + nchunk - 1) / nchunk) + 1) & ~1;   // even, so chunk parity is uniform
@@ -782,6 +809,9 @@ static int launch_frames_bwd(const float *g_audio, const uint64_t *phi, const ui
     dim3 grid((T + fr - 1) / fr, B);
     auto kernel = rc ? harmonic_frames_bwd_w_x2_kernel<true> : harmonic_frames_bwd_w_x2_kernel<false>;
     if (smem > 48 * 1024) cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    if (programmatic)
+        return ddsp_launch_programmatic(kernel, grid, dim3(kBwdThreads), smem, st, g_audio, phi, delta, d_weights, T, H,
+                                        bs, fr, nchunk, clen, rc ? *rc : RawControlsGrad{});
     kernel<<<grid, kBwdThreads, smem, st>>>(g_audio, phi, delta, d_weights, T, H, bs, fr, nchunk, clen,
                                             rc ? *rc : RawControlsGrad{});
     return ddsp_launch_status();
@@ -807,6 +837,18 @@ extern "C" int ddsp_b200_harmonic_frames_raw_bwd(const float *g_audio, const flo
     RawControlsGrad rc{amp_raw, dist_raw, f0, amp_stride, dist_stride, sample_rate * 0.5f,
                        d_amp_raw, d_dist_raw, d_amp_stride, d_dist_stride};
     return launch_frames_bwd(g_audio, phi, delta, nullptr, &rc, B, T, H, block_size, (cudaStream_t)stream);
+}
+
+int ddsp_pair_bank_bwd(const float *g_audio, const float *amp_raw, int64_t amp_stride, const float *dist_raw,
+                       int64_t dist_stride, const float *f0, const uint64_t *phi, const uint64_t *delta,
+                       float *d_amp_raw, int64_t d_amp_stride, float *d_dist_raw, int64_t d_dist_stride, int B, int T,
+                       int H, int block_size, float sample_rate, cudaStream_t st) {
+    DDSP_REQUIRE(g_audio && amp_raw && dist_raw && f0 && phi && delta && d_amp_raw && d_dist_raw);
+    DDSP_REQUIRE(B > 0 && B <= 65535 && T > 0 && H > 0 && block_size > 0);
+    DDSP_REQUIRE(amp_stride >= 1 && dist_stride >= H && d_amp_stride >= 1 && d_dist_stride >= H);
+    RawControlsGrad rc{amp_raw, dist_raw, f0, amp_stride, dist_stride, sample_rate * 0.5f,
+                       d_amp_raw, d_dist_raw, d_amp_stride, d_dist_stride};
+    return launch_frames_bwd(g_audio, phi, delta, nullptr, &rc, B, T, H, block_size, st, true);
 }
 
 extern "C" int ddsp_b200_harmonic_frames_bwd_f0(const float *g_audio, const float *weights,

@@ -386,11 +386,15 @@ struct Noise2Layout {         // per-row shared areas of the second-generation k
     __host__ __device__ int yf() const { return NBq + F + xs_len + bs; }
 };
 
+// PAIR: launched first of the synth pair (ddsp_b200_synth_pair_fwd / _bwd); the oscillator bank is its programmatic
+// dependent and is dispatched beside it as soon as every CTA has started here
+template <bool PAIR>
 __global__ void __launch_bounds__(kN2Threads)
 filtered_noise2_fwd_kernel(const float *__restrict__ mags, const float *__restrict__ noise,
                            const float *__restrict__ add, const float *__restrict__ design,
                            float *__restrict__ out, int64_t rows, int NB, int bs, int RPC, int apply_scale,
                            float bias) {
+    if (PAIR) asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
     extern __shared__ __align__(16) float smem[];
     const Noise2Layout L(NB, bs);
     const int half = L.half, F = L.F;
@@ -494,11 +498,13 @@ filtered_noise2_fwd_kernel(const float *__restrict__ mags, const float *__restri
     }
 }
 
+template <bool PAIR>
 __global__ void __launch_bounds__(kN2Threads)
 filtered_noise2_bwd_kernel(const float *__restrict__ g_out, const float *__restrict__ noise,
                            const float *__restrict__ mags_raw, const float *__restrict__ design,
                            float *__restrict__ d_mags, int64_t rows, int NB, int bs, int RPC,
                            int apply_scale, float bias) {
+    if (PAIR) asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
     extern __shared__ __align__(16) float smem[];
     const Noise2Layout L(NB, bs);
     const int half = L.half, F = L.F, NBq = L.NBq;
@@ -643,6 +649,26 @@ static bool noise2_cfg(int64_t rows, int NB, int bs, bool bwd, int *rpc, size_t 
     return true;
 }
 
+// The synth pair (ddsp_b200_synth_pair_fwd / _bwd): exactly k persistent CTAs per SM, launched before the oscillator
+// bank, whose CTAs take the rest of each SM.  The k CTAs keep at most half of the SM's shared memory, and every CTA
+// gets at least one full sweep of RPC rows (fewer rows: the pair does not apply).  A row's arithmetic does not depend
+// on RPC or on the grid, so the pair computes the same bits as the standalone launch.
+constexpr int kPairCtasFwd = 1, kPairCtasBwd = 2;        // per SM; chosen with tools/synth_overlap.py
+
+static bool noise2_pair_cfg(int64_t rows, int NB, int bs, bool bwd, int k, int *rpc, size_t *smem, int *grid) {
+    if (k < 1 || k > 2 || NB < 5 || (NB - 1) % 4 != 0 || bs % 4 != 0 || bs < 2 * (NB - 1)) return false;
+    const Noise2Layout L(NB, bs);
+    const size_t fixed = (bwd ? (size_t)L.F * L.NBq : (size_t)NB * L.F) * sizeof(float);
+    const size_t budget = (size_t)112 * 1024 / k;
+    int r = 16;
+    while (r > 1 && fixed + (size_t)r * L.stride * sizeof(float) > budget) r >>= 1;
+    *smem = fixed + (size_t)r * L.stride * sizeof(float);
+    if (*smem > budget || rows < (int64_t)k * DDSP_SM_COUNT * r) return false;
+    *rpc = r;
+    *grid = k * DDSP_SM_COUNT;
+    return true;
+}
+
 extern "C" int64_t ddsp_b200_noise_design_size(int NB) {
     if (NB < 2) return 0;
     const int F = 2 * (NB - 1), NBq = (NB + 3) & ~3;
@@ -664,9 +690,9 @@ extern "C" int ddsp_b200_filtered_noise_fwd(const float *mags, const float *nois
     size_t smem;
     if (design && noise2_cfg(rows, NB, block_size, false, &rpc, &smem, &grid)) {
         if (smem > 48 * 1024)
-            cudaFuncSetAttribute(filtered_noise2_fwd_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
+            cudaFuncSetAttribute(filtered_noise2_fwd_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                  (int)smem);
-        filtered_noise2_fwd_kernel<<<grid, kN2Threads, smem, (cudaStream_t)stream>>>(
+        filtered_noise2_fwd_kernel<false><<<grid, kN2Threads, smem, (cudaStream_t)stream>>>(
             mags, noise, add, design, out, rows, NB, block_size, rpc, apply_scale, bias);
         return ddsp_launch_status();
     }
@@ -690,9 +716,9 @@ extern "C" int ddsp_b200_filtered_noise_bwd(const float *g_out, const float *noi
     size_t smem;
     if (design && noise2_cfg(rows, NB, block_size, true, &rpc, &smem, &grid)) {
         if (smem > 48 * 1024)
-            cudaFuncSetAttribute(filtered_noise2_bwd_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
+            cudaFuncSetAttribute(filtered_noise2_bwd_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                  (int)smem);
-        filtered_noise2_bwd_kernel<<<grid, kN2Threads, smem, (cudaStream_t)stream>>>(
+        filtered_noise2_bwd_kernel<false><<<grid, kN2Threads, smem, (cudaStream_t)stream>>>(
             g_out, noise, mags_raw, design, d_mags, rows, NB, block_size, rpc, apply_scale, bias);
         return ddsp_launch_status();
     }
@@ -704,4 +730,83 @@ extern "C" int ddsp_b200_filtered_noise_bwd(const float *g_out, const float *noi
     filtered_noise_bwd_kernel<<<grid, kNoiseThreads, smem, (cudaStream_t)stream>>>(
         g_out, noise, mags_raw, d_mags, rows, NB, block_size, rpc, apply_scale, bias);
     return ddsp_launch_status();
+}
+
+extern "C" int ddsp_b200_synth_pair_supported(int B, int T, int H, int NB, int block_size, int ctas_per_sm) {
+    if (B < 1 || B > 65535 || T < 1 || ctas_per_sm < 0 || ctas_per_sm > 2) return 0;
+    if (!ddsp_pair_bank_supported(T, H, block_size)) return 0;
+    const int64_t rows = (int64_t)B * T;
+    int rpc, grid;
+    size_t smem;
+    return noise2_pair_cfg(rows, NB, block_size, false, ctas_per_sm ? ctas_per_sm : kPairCtasFwd, &rpc, &smem, &grid) &&
+           noise2_pair_cfg(rows, NB, block_size, true, ctas_per_sm ? ctas_per_sm : kPairCtasBwd, &rpc, &smem, &grid);
+}
+
+// The noise kernel's shared-memory carveout is set to the largest, so that the SM configuration it is dispatched with
+// also has room for the bank's CTAs.
+template <typename K>
+static void pair_noise_attributes(K kernel, size_t smem) {
+    cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    cudaFuncSetAttribute(kernel, cudaFuncAttributePreferredSharedMemoryCarveout, (int)cudaSharedmemCarveoutMaxShared);
+}
+
+// The noise's consumer (the reverb's first pass in the forward, the end of the step in the backward) comes after
+// this call on `stream`.  The bank is the noise kernel's programmatic dependent, and that edge does not make "bank
+// finished" imply "noise finished": `event` is recorded after the noise launch and waited for after the bank's, so
+// that everything queued later also waits for the noise kernel to complete.
+static int pair_join(int status, cudaEvent_t event, cudaStream_t st) {
+    if (status) return status;
+    const cudaError_t e = cudaStreamWaitEvent(st, event, 0);
+    return e == cudaSuccess ? DDSP_B200_OK : (int)e;
+}
+
+extern "C" int ddsp_b200_synth_pair_fwd(const float *amp_raw, int64_t amp_stride, const float *dist_raw,
+                                        int64_t dist_stride, const float *f0, const double *phase0, uint64_t *phi,
+                                        uint64_t *delta, double *phase_end, float *amps, float *weights, float *audio,
+                                        const float *mags_raw, const float *noise, const float *design,
+                                        float *noise_out, int B, int T, int H, int NB, int block_size,
+                                        double sample_rate, float bias, int ctas_per_sm, void *event, void *stream) {
+    DDSP_REQUIRE(mags_raw && noise && design && noise_out && event && B > 0 && T > 0 && sample_rate > 0);
+    if (!ddsp_b200_synth_pair_supported(B, T, H, NB, block_size, ctas_per_sm)) return DDSP_B200_EUNSUPPORTED;
+    const int64_t rows = (int64_t)B * T;
+    int rpc, grid;
+    size_t smem;
+    noise2_pair_cfg(rows, NB, block_size, false, ctas_per_sm ? ctas_per_sm : kPairCtasFwd, &rpc, &smem, &grid);
+    cudaStream_t st = (cudaStream_t)stream;
+    pair_noise_attributes(filtered_noise2_fwd_kernel<true>, smem);
+    filtered_noise2_fwd_kernel<true><<<grid, kN2Threads, smem, st>>>(mags_raw, noise, nullptr, design, noise_out, rows,
+                                                                     NB, block_size, rpc, 1, bias);
+    int s = ddsp_launch_status();
+    if (s) return s;
+    const cudaError_t e = cudaEventRecord((cudaEvent_t)event, st);
+    if (e != cudaSuccess) return (int)e;
+    s = ddsp_pair_bank_fwd(amp_raw, amp_stride, dist_raw, dist_stride, f0, phase0, phi, delta, phase_end, amps, weights,
+                           audio, B, T, H, block_size, sample_rate, st);
+    return pair_join(s, (cudaEvent_t)event, st);
+}
+
+extern "C" int ddsp_b200_synth_pair_bwd(const float *g_audio, const float *g_noise, const float *amp_raw,
+                                        int64_t amp_stride, const float *dist_raw, int64_t dist_stride, const float *f0,
+                                        const uint64_t *phi, const uint64_t *delta, float *d_amp_raw,
+                                        int64_t d_amp_stride, float *d_dist_raw, int64_t d_dist_stride,
+                                        const float *mags_raw, const float *noise, const float *design, float *d_mags,
+                                        int B, int T, int H, int NB, int block_size, float sample_rate, float bias,
+                                        int ctas_per_sm, void *event, void *stream) {
+    DDSP_REQUIRE(g_noise && mags_raw && noise && design && d_mags && event && B > 0 && T > 0);
+    if (!ddsp_b200_synth_pair_supported(B, T, H, NB, block_size, ctas_per_sm)) return DDSP_B200_EUNSUPPORTED;
+    const int64_t rows = (int64_t)B * T;
+    int rpc, grid;
+    size_t smem;
+    noise2_pair_cfg(rows, NB, block_size, true, ctas_per_sm ? ctas_per_sm : kPairCtasBwd, &rpc, &smem, &grid);
+    cudaStream_t st = (cudaStream_t)stream;
+    pair_noise_attributes(filtered_noise2_bwd_kernel<true>, smem);
+    filtered_noise2_bwd_kernel<true><<<grid, kN2Threads, smem, st>>>(g_noise, noise, mags_raw, design, d_mags, rows, NB,
+                                                                     block_size, rpc, 1, bias);
+    int s = ddsp_launch_status();
+    if (s) return s;
+    const cudaError_t e = cudaEventRecord((cudaEvent_t)event, st);
+    if (e != cudaSuccess) return (int)e;
+    s = ddsp_pair_bank_bwd(g_audio, amp_raw, amp_stride, dist_raw, dist_stride, f0, phi, delta, d_amp_raw, d_amp_stride,
+                           d_dist_raw, d_dist_stride, B, T, H, block_size, sample_rate, st);
+    return pair_join(s, (cudaEvent_t)event, st);
 }

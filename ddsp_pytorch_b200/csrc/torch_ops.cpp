@@ -451,6 +451,86 @@ Tensor noise_bwd(const Tensor &g_, const Tensor &noise_, const c10::optional<Ten
     return d_mags;
 }
 
+// ---------------------------------------------------------------------------------------- a3+a6 beside a7+a8+a9
+// The oscillator bank from raw controls and the fused filtered noise as one pair of launches on the current stream
+// (ddsp_b200_synth_pair_fwd / _bwd).  The pair's join event is one per device; the lock keeps its record / wait
+// inside one call.
+std::mutex pair_mu;
+
+cudaEvent_t pair_event(const at::Device &dev) {
+    static std::map<int, cudaEvent_t> events;
+    auto it = events.find((int)dev.index());
+    if (it != events.end()) return it->second;
+    cudaEvent_t e = nullptr;
+    TORCH_CHECK(cudaEventCreateWithFlags(&e, cudaEventDisableTiming) == cudaSuccess, "ddsp_b200: synth pair event");
+    events[(int)dev.index()] = e;
+    return e;
+}
+
+int64_t synth_pair_supported(int64_t B, int64_t T, int64_t H, int64_t NB, int64_t block_size, int64_t ctas_per_sm) {
+    return ddsp_b200_synth_pair_supported((int)B, (int)T, (int)H, (int)NB, (int)block_size, (int)ctas_per_sm);
+}
+
+// -> (harmonic audio (B,T*bs,1), noise (B,T*bs,1), phi, delta)
+std::tuple<Tensor, Tensor, Tensor, Tensor> synth_pair_fwd(const Tensor &amp_raw_, const Tensor &dist_raw_,
+                                                          const Tensor &f0_, const Tensor &mags_raw_,
+                                                          const Tensor &noise_, int64_t block_size, double sample_rate,
+                                                          double bias, int64_t ctas_per_sm) {
+    RawViews v = raw_views(amp_raw_, dist_raw_);
+    Tensor f0 = prep(f0_, "f0"), mags = prep(mags_raw_, "magnitudes"), noise = prep(noise_, "noise");
+    const int64_t B = v.B, T = v.T, H = v.H;
+    TORCH_CHECK(f0.numel() == B * T, "synth_pair_fwd: f0 must be (B,T,1)");
+    TORCH_CHECK(mags.dim() == 3 && mags.size(0) == B && mags.size(1) == T && noise.dim() == 3 && noise.size(0) == B &&
+                    noise.size(1) == T && noise.size(2) == block_size,
+                "synth_pair_fwd: magnitudes (B,T,NB) and noise (B,T,block) expected");
+    const int64_t NB = mags.size(2);
+    c10::cuda::CUDAGuard guard(f0.device());
+    auto opt = f0.options();
+    Tensor phi = at::empty({B, T}, opt.dtype(at::kLong)), delta = at::empty({B, T}, opt.dtype(at::kLong));
+    Tensor audio = at::empty({B, T * block_size, 1}, opt), out = at::empty({B, T * block_size, 1}, opt);
+    Tensor amps = at::empty({B, T, 1}, opt), weights = at::empty({B, T, H}, opt);
+    Tensor design = noise_design_table(f0.device(), NB);
+    std::lock_guard<std::mutex> lock(pair_mu);
+    check(ddsp_b200_synth_pair_fwd(v.amp, v.amp_stride, v.dst, v.dist_stride, fp(f0), nullptr,
+                                   (uint64_t *)phi.data_ptr<int64_t>(), (uint64_t *)delta.data_ptr<int64_t>(), nullptr,
+                                   fpm(amps), fpm(weights), fpm(audio), fp(mags), fp(noise), fp(design), fpm(out),
+                                   (int)B, (int)T, (int)H, (int)NB, (int)block_size, sample_rate, (float)bias,
+                                   (int)ctas_per_sm, pair_event(f0.device()), cur_stream()),
+          "synth_pair_fwd");
+    return {audio, out, phi, delta};
+}
+
+// -> (d_amp_raw (B,T,1), d_dist_raw (B,T,H), d_mags_raw (B,T,NB))
+std::tuple<Tensor, Tensor, Tensor> synth_pair_bwd(const Tensor &g_audio_, const Tensor &g_noise_,
+                                                  const Tensor &amp_raw_, const Tensor &dist_raw_, const Tensor &f0_,
+                                                  const Tensor &phi, const Tensor &delta, const Tensor &mags_raw_,
+                                                  const Tensor &noise_, int64_t block_size, double sample_rate,
+                                                  double bias, int64_t ctas_per_sm) {
+    RawViews v = raw_views(amp_raw_, dist_raw_);
+    Tensor g = prep(g_audio_, "grad_audio"), gn = prep(g_noise_, "grad_noise"), f0 = prep(f0_, "f0"),
+           mags = prep(mags_raw_, "magnitudes"), noise = prep(noise_, "noise");
+    const int64_t B = v.B, T = v.T, H = v.H, NB = mags.size(-1);
+    TORCH_CHECK(g.numel() == B * T * block_size && gn.numel() == B * T * block_size && f0.numel() == B * T &&
+                    mags.numel() == B * T * NB && noise.numel() == B * T * block_size,
+                "synth_pair_bwd: shape mismatch");
+    TORCH_CHECK(phi.is_cuda() && phi.scalar_type() == at::kLong && phi.is_contiguous() &&
+                    delta.is_cuda() && delta.scalar_type() == at::kLong && delta.is_contiguous() &&
+                    phi.numel() == B * T && delta.numel() == B * T,
+                "synth_pair_bwd: bad phase workspace");
+    c10::cuda::CUDAGuard guard(g.device());
+    Tensor da = at::empty({B, T, 1}, g.options()), dd = at::empty({B, T, H}, g.options());
+    Tensor dm = at::empty({B, T, NB}, g.options());
+    Tensor design = noise_design_table(g.device(), NB);
+    std::lock_guard<std::mutex> lock(pair_mu);
+    check(ddsp_b200_synth_pair_bwd(fp(g), fp(gn), v.amp, v.amp_stride, v.dst, v.dist_stride, fp(f0),
+                                   (const uint64_t *)phi.data_ptr<int64_t>(), (const uint64_t *)delta.data_ptr<int64_t>(),
+                                   fpm(da), 1, fpm(dd), H, fp(mags), fp(noise), fp(design), fpm(dm), (int)B, (int)T,
+                                   (int)H, (int)NB, (int)block_size, (float)sample_rate, (float)bias, (int)ctas_per_sm,
+                                   pair_event(g.device()), cur_stream()),
+          "synth_pair_bwd");
+    return {da, dd, dm};
+}
+
 // ---------------------------------------------------------------------------------------- a9, a10
 struct ConvPlan {
     int n1, n2;
@@ -1050,6 +1130,9 @@ TORCH_LIBRARY(ddsp_b200, m) {
     m.def("amp_to_ir_bwd(Tensor d_ir, int n_bands) -> Tensor");
     m.def("noise_fwd(Tensor magnitudes, Tensor noise, Tensor? add, bool apply_scale, float bias) -> Tensor");
     m.def("noise_bwd(Tensor grad_out, Tensor noise, Tensor? magnitudes_raw, int n_bands, bool apply_scale, float bias) -> Tensor");
+    m.def("synth_pair_supported(int B, int T, int n_harmonic, int n_bands, int block_size, int ctas_per_sm=0) -> int", synth_pair_supported);
+    m.def("synth_pair_fwd(Tensor amplitudes, Tensor harmonic_distribution, Tensor f0, Tensor magnitudes_raw, Tensor noise, int block_size, float sample_rate, float bias, int ctas_per_sm=0) -> (Tensor, Tensor, Tensor, Tensor)");
+    m.def("synth_pair_bwd(Tensor grad_audio, Tensor grad_noise, Tensor amplitudes, Tensor harmonic_distribution, Tensor f0, Tensor phi, Tensor delta, Tensor magnitudes_raw, Tensor noise, int block_size, float sample_rate, float bias, int ctas_per_sm=0) -> (Tensor, Tensor, Tensor)");
     m.def("fftconv_spectrum(Tensor kernel, int n_signal) -> Tensor");
     m.def("fftconv_fwd(Tensor signal, Tensor kernel, bool keep_transforms, Tensor? hspec=None, Tensor? signal2=None) -> (Tensor, Tensor, Tensor)");
     m.def("fftconv_bwd(Tensor grad_out, Tensor signal, Tensor kernel, Tensor? work_x, Tensor? hspec, bool need_signal, bool need_kernel) -> (Tensor, Tensor)");
@@ -1088,6 +1171,8 @@ TORCH_LIBRARY_IMPL(ddsp_b200, CUDA, m) {
     m.impl("amp_to_ir_bwd", amp_to_ir_bwd);
     m.impl("noise_fwd", noise_fwd);
     m.impl("noise_bwd", noise_bwd);
+    m.impl("synth_pair_fwd", synth_pair_fwd);
+    m.impl("synth_pair_bwd", synth_pair_bwd);
     m.impl("fftconv_spectrum", fftconv_spectrum);
     m.impl("fftconv_fwd", fftconv_fwd);
     m.impl("fftconv_bwd", fftconv_bwd);

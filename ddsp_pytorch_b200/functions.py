@@ -322,6 +322,36 @@ class FilteredNoiseFused(torch.autograd.Function):
         return d_raw, None, (g if ctx.needs_input_grad[2] else None), None
 
 
+class SynthPair(torch.autograd.Function):
+    """HarmonicFromRaw (split form, no phase carry) and FilteredNoiseFused (no ``add``) as one node: amp_raw (B,T,1),
+    dist_raw (B,T,H), mag_raw (B,T,NB), f0 (B,T,1), noise draw (B,T,bs) -> (harmonic (B,T*bs,1), noise (B,T*bs,1)).
+    Each direction is one ``synth_pair_*`` call: the noise kernel as persistent CTAs with the oscillator bank launched
+    beside it, same bits as the two Functions.  One node also fixes the backward's order (noise first, then the bank
+    as its dependent), which autograd's order between two nodes would not.  ``ctas_per_sm``: noise CTAs per SM (0 =
+    the library's choice); see ``synth_pair_supported``."""
+
+    @staticmethod
+    def forward(ctx, amp_raw, dist_raw, mag_raw, f0, noise, block_size, sample_rate, bias, ctas_per_sm=0):
+        ctx.cfg = (int(block_size), float(sample_rate), float(bias), int(ctas_per_sm))
+        audio, noise_out, phi, delta = _ops.synth_pair_fwd(amp_raw, dist_raw, f0, mag_raw, noise, *ctx.cfg)
+        ctx.save_for_backward(amp_raw, dist_raw, mag_raw, f0, noise, phi, delta)
+        return audio, noise_out
+
+    @staticmethod
+    @once_differentiable
+    def backward(ctx, g_audio, g_noise):
+        amp_raw, dist_raw, mag_raw, f0, noise, phi, delta = ctx.saved_tensors
+        da, dd, dm = _ops.synth_pair_bwd(g_audio, g_noise, amp_raw, dist_raw, f0, phi, delta, mag_raw, noise, *ctx.cfg)
+        return da.view_as(amp_raw), dd.view_as(dist_raw), dm.view_as(mag_raw), None, None, None, None, None, None
+
+
+def synth_pair_supported(shapes, ctas_per_sm: int = 0) -> bool:
+    """Whether SynthPair runs at these SynthShapes: the bank takes its phase scan inside its launch and every noise CTA
+    gets at least one full sweep of frames (small batches leave the noise grid part empty)."""
+    s = shapes
+    return bool(_ops.synth_pair_supported(s.batch, s.frames, s.n_harmonic, s.n_bands, s.block_size, int(ctas_per_sm)))
+
+
 class FFTConvolve(torch.autograd.Function):
     """core.py:169-176 on 2-D (rows, n) operands; kernel rows 1 (shared) or equal to signal rows.
     When a gradient will be needed the forward keeps the transform of the signal and the kernel spectrum

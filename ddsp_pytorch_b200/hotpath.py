@@ -47,6 +47,10 @@ class SynthStep:
         self._graph = None
         self._graph_fwd = None
         self._dist = None                  # set by enable_grad_allreduce (data-parallel training config)
+        # the two synthesisers as one SynthPair node (noise CTAs per SM, 0 = the library's choice) where it applies,
+        # else on two streams (None)
+        self._pair_ctas = 0 if (core.harmonic_raw_supported(s.n_harmonic, s.block_size) and
+                                F_.synth_pair_supported(s)) else None
 
     def _offsets(self):
         off, out = 0, []
@@ -129,27 +133,34 @@ class SynthStep:
             leaves = [i["amp_raw"], i["dist_raw"], i["mag_raw"]]
             if self.reverb is not None:
                 leaves += [self.reverb.noise, self.reverb.decay, self.reverb.wet]
-        # The noise branch and the harmonic branch are independent until the mix (decoder.py:121): run the
-        # noise branch on a side stream.  Autograd replays each node's backward on its forward stream, so the
-        # two backward branches overlap as well; under capture both become parallel graph branches.
+        # The noise branch and the harmonic branch are independent until the mix (decoder.py:121).  Where the pair
+        # applies, both synthesisers are one SynthPair node on the current stream: the noise kernel's persistent CTAs
+        # and the oscillator bank share every SM in each direction.  Elsewhere the noise branch runs on a side stream
+        # (autograd replays each node's backward on its forward stream, so the two backward branches overlap as well;
+        # under capture both become parallel graph branches).
         cur = torch.cuda.current_stream()
         side = self._side_stream
         kernel = hspec = None
+        noise = None
         side.wait_stream(cur)
         with torch.cuda.stream(side):
             if self.reverb is not None:
                 # the reverb's impulse depends on the reverb parameters only: it is built, and its spectrum computed,
                 # on the side stream.  Autograd replays a node's backward on its forward stream, so the impulse's
-                # backward (two small launches at the very end of the step) also lands beside the oscillator bank's
+                # backward (two small launches at the very end of the step) also lands beside the synthesisers'
                 # backward instead of after it
                 impulse = F_.ReverbImpulse.apply(leaves[3], leaves[4], leaves[5], self.reverb.t)
                 taps = min(s.samples, s.reverb_length)
                 kernel = impulse.reshape(1, s.reverb_length)[:, :taps]
                 hspec = F_._ops.fftconv_spectrum(kernel.detach(), s.samples)
-            # FilteredNoise.get_controls + forward in one launch
-            noise = F_.FilteredNoiseFused.apply(leaves[2], i["noise"], None, -5.0)
-        # HarmonicSynth.get_controls + forward in one launch (the controls are the oscillator bank's prologue)
-        if core.harmonic_raw_supported(s.n_harmonic, s.block_size):
+            if self._pair_ctas is None:
+                # FilteredNoise.get_controls + forward in one launch
+                noise = F_.FilteredNoiseFused.apply(leaves[2], i["noise"], None, -5.0)
+        if self._pair_ctas is not None:
+            harmonic, noise = F_.SynthPair.apply(leaves[0], leaves[1], leaves[2], i["pitch"], i["noise"], s.block_size,
+                                                 s.sample_rate, -5.0, self._pair_ctas)
+        elif core.harmonic_raw_supported(s.n_harmonic, s.block_size):
+            # HarmonicSynth.get_controls + forward in one launch (the controls are the oscillator bank's prologue)
             harmonic = core.harmonic_synth_from_raw(leaves[0], leaves[1], i["pitch"], s.block_size, s.sample_rate)[0]
         else:
             _, _, weights = F_.HarmonicControlsWeights.apply(leaves[0], leaves[1], i["pitch"], float(s.sample_rate))

@@ -151,6 +151,29 @@ int ddsp_b200_filtered_noise_bwd(const float *g_out, const float *noise, const f
                                  const float *design, float *d_mags, int64_t rows, int NB,
                                  int block_size, int apply_scale, float bias, void *stream);
 
+/* ---- a3+a6 beside a7+a8+a9: the oscillator bank and the filtered noise as one pair of launches ------------------
+ * ddsp_b200_harmonic_frames_raw_scan_fwd and ddsp_b200_filtered_noise_fwd (apply_scale = 1, add = NULL) in one call,
+ * and their backward (ddsp_b200_filtered_noise_bwd with apply_scale = 1, ddsp_b200_harmonic_frames_raw_bwd); same
+ * arguments, same bits.  The noise kernel runs as a fixed number of persistent CTAs per SM and the bank is launched
+ * as its programmatic dependent on the same stream, so the two run on every SM at once (the bank is bound by the FMA
+ * pipe, the noise by shared-memory wavefronts).  Work queued on `stream` after the call waits for both kernels.
+ * event: a cudaEvent_t created by the caller (cudaEventDisableTiming), recorded and waited for on `stream` inside the
+ * call; one call at a time per event.  ctas_per_sm: noise CTAs per SM (1 or 2; 0 = the library's choice per direction).
+ * Supported when the bank takes the scan inside its launch and every noise CTA gets at least one full sweep of rows
+ * (ddsp_b200_synth_pair_supported); else DDSP_B200_EUNSUPPORTED: use the two entry points on two streams.       */
+int ddsp_b200_synth_pair_supported(int B, int T, int H, int NB, int block_size, int ctas_per_sm);
+int ddsp_b200_synth_pair_fwd(const float *amp_raw, int64_t amp_stride, const float *dist_raw, int64_t dist_stride,
+                             const float *f0, const double *phase0, uint64_t *phi, uint64_t *delta, double *phase_end,
+                             float *amps, float *weights, float *audio, const float *mags_raw, const float *noise,
+                             const float *design, float *noise_out, int B, int T, int H, int NB, int block_size,
+                             double sample_rate, float bias, int ctas_per_sm, void *event, void *stream);
+int ddsp_b200_synth_pair_bwd(const float *g_audio, const float *g_noise, const float *amp_raw, int64_t amp_stride,
+                             const float *dist_raw, int64_t dist_stride, const float *f0, const uint64_t *phi,
+                             const uint64_t *delta, float *d_amp_raw, int64_t d_amp_stride, float *d_dist_raw,
+                             int64_t d_dist_stride, const float *mags_raw, const float *noise, const float *design,
+                             float *d_mags, int B, int T, int H, int NB, int block_size, float sample_rate, float bias,
+                             int ctas_per_sm, void *event, void *stream);
+
 /* ---- FFT tables (caller-owned constant tables) --------------------------------------------- */
 /* table[m] = (cos, -sin)(2*pi*m/n), m in [0,n): n float2 = 2n floats; n a power of two.  One
  * table of size n serves every transform whose size divides n (read with stride n/size).       */
